@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm (oracle port on host cores)
+    python bench.py ... --dump-outputs DIR                    # + the last timed turn's outputs as DIR/<name>.npy
 
 Workload (config.workload): BASELINE config 4's per-GPU shard -- 131072 lock-step environments per
 GPU (1M environments at 8 GPUs), full-rules random self-play: per env turn = Philox dice ->
@@ -208,7 +209,7 @@ def python_reference_rates(cores, seconds=5.0):
     if _pyref_setup() is None:
         return None
     import multiprocessing as mp
-    out = {"cores": cores, "seconds_per_row": seconds, "source": "baseline/_ref (unmodified /root/reference files, gymnasium stubbed)"}
+    out = {"cores": cores, "seconds_per_row": seconds, "source": "baseline/_ref (unmodified files of the original gym-narde, gymnasium stubbed)"}
     ctx = mp.get_context("spawn")
     with ctx.Pool(cores) as pool:
         for mode, key in (("step", "NardeEnv_step_valid_random"), ("enum", "pair_enumeration_plus_step")):
@@ -358,6 +359,9 @@ def run_cuda_arm(args):
     wall_ms = 1e3 * (time.perf_counter() - t_wall0)
     clocks = sampler.stop()
     dstats = (env.stats - stats0).cpu().tolist()
+    dumped = None
+    if args.dump_outputs and rank == 0:      # before any further turn overwrites the last timed one
+        dumped = dump_step_outputs(env, args.dump_outputs)
     total_ms = sum(ms)
     A = dstats[5] / float(E * K * R)
     # stored list entries per env turn = min(count, cap): what the kernel really writes (roofline bytes)
@@ -605,6 +609,8 @@ def run_cuda_arm(args):
             line["policy_broadcast_ms"] = bcast_ms
         if cross is not None:
             line["cross_rank_shard_check"] = cross
+        if dumped is not None:
+            line["dumped_outputs"] = dumped
         if cfg5 is not None:
             line["config5_afterstate_scoring"] = cfg5
         line["back_to_back"] = {"ms_per_turn": ms_b2b, "value_rank0": E / (ms_b2b * 1e-3), "turns": n_b2b,
@@ -623,6 +629,31 @@ def run_cuda_arm(args):
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ENVS = 65536    # 832 bytes of float32 outputs per env: a sample of this many envs stays under 64 MB
+
+
+def dump_step_outputs(env, out_dir):
+    """--dump-outputs: what the last VecNardeEnv.step() returned, as float32 DIR/<name>.npy.  step() returns the env's
+    persistent output buffers, so right after the timed loop they hold the last timed turn.  Every array keeps the same
+    rows: all envs, or a fixed seeded sample of DUMP_ENVS of them.  The arguments fix the inputs (seed, env ids, number
+    of turns), so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    torch = env.torch
+    n = env.num_envs
+    rows = np.arange(n) if n <= DUMP_ENVS else np.sort(np.random.default_rng(SEED).choice(n, DUMP_ENVS, replace=False))
+    idx = torch.from_numpy(rows).to(env.device)
+    info = env.info
+    arrays = {"obs": env.obs, "reward": env.reward, "terminated": env.terminated, "truncated": env.truncated,
+              "dice": info["dice"], "counts": info["counts"]}
+    arrays = {k: v[idx].to(torch.float32).cpu().numpy() for k, v in arrays.items()}
+    # a turn action is four u16 half-moves (include/narde_b200.h): column k holds bits 16k..16k+15, exact in float32
+    arrays["chosen"] = info["chosen"][idx].cpu().numpy().view(np.uint16).reshape(-1, 4).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    return {"dir": out_dir, "turn": env.step_count, "envs": int(len(rows)), "arrays": sorted(arrays)}
 
 
 def parity_and_cpu_baseline(torch, env, args, cfg3):
@@ -813,7 +844,11 @@ def main():
     ap.add_argument("--no-python-reference", action="store_true")
     ap.add_argument("--turns-per-step", type=int, default=128,
                     help="lock-step turns (graph replays, each timed on its own with a flushed L2) that make one 'step'")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what VecNardeEnv.step() returned on the last timed turn as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the CUDA path's outputs; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -1,9 +1,10 @@
-"""Loads the REAL Python reference (read-only, /root/reference) -- TEST INFRASTRUCTURE ONLY.
+"""Loads the REAL Python reference (the original gym-narde) -- TEST INFRASTRUCTURE ONLY.
 
-The reference needs `gymnasium`, which is not installed in this image; a minimal stub of the
-few names it touches (Env, spaces.Box/Discrete/Tuple, envs.registration.register) is injected
-into sys.modules when the real package is absent.  Nothing here is available on the GPU box
-(no /root/reference there): callers must check `available()` and skip.
+The original is not part of this repository: it is read from NARDE_REFERENCE_ROOT, or else from
+baseline/_ref (vendored there by baseline/fetch_ref.py).  Where neither holds it, callers must
+check `available()` and skip.
+The reference needs `gymnasium`; when the real package is absent, a minimal stub of the few names
+it touches (Env, spaces.Box/Discrete/Tuple, envs.registration.register) is injected into sys.modules.
 
 `injected_dice(stream)` replays an explicit dice stream through the reference by patching
 numpy.random.randint, which is the only RNG call the reference env makes
@@ -19,7 +20,8 @@ from unittest import mock
 
 import numpy as np
 
-REF_ROOT = os.environ.get("NARDE_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("NARDE_REFERENCE_ROOT") or os.path.join(
+    os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
 
 
 def available() -> bool:

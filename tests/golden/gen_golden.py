@@ -1,7 +1,6 @@
-"""Generates the committed golden fixtures from the REAL reference (/root/reference).
-
-Run in the build container only (the GPU box has no /root/reference):
-    python tests/golden/gen_golden.py
+"""Generates the committed golden fixtures from the REAL reference (the original gym-narde, which is not part of
+this repository; oracle/ref_loader.py finds it through NARDE_REFERENCE_ROOT or baseline/_ref):
+    NARDE_REFERENCE_ROOT=<gym-narde checkout> python tests/golden/gen_golden.py
 Outputs (small JSON files next to this script):
   ref_valid_moves.json   Narde.get_valid_moves(roll, player) ordered lists (narde.py:58-92)
   ref_step_traces.json   NardeEnv.reset/step traces with an injected dice stream (narde_env.py:27-120)

@@ -1,7 +1,8 @@
 """GPU (-m gpu): the reference's OWN tests and caller scripts, unmodified, against this repo's env.
 
-baseline/fetch_ref.py vendors the untouched reference files into baseline/_ref (git-ignored; it travels to the GPU
-box).  tests/refsuite_runner.py runs them in a fresh process twice: on the real reference env, and with
+The original is not part of this repository: baseline/fetch_ref.py vendors its untouched files from a checkout into
+baseline/_ref (git-ignored), and these tests skip without them.  tests/refsuite_runner.py runs them in a fresh
+process twice: on the real reference env, and with
 `gym_narde` aliased to the GPU facade (gym_narde_b200.envs.NardeEnv / Narde through the C ABI).
 
   * north star: tests/test_move_validation.py and tests/test_doubles_sequence.py pass against the new env
@@ -24,7 +25,9 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 RUNNER = os.path.join(ROOT, "tests", "refsuite_runner.py")
 HAVE_REF = os.path.isfile(os.path.join(ROOT, "baseline", "_ref", "gym_narde", "envs", "narde.py"))
-needs_ref = pytest.mark.skipif(not HAVE_REF, reason="baseline/_ref not vendored (run baseline/fetch_ref.py where /root/reference exists)")
+needs_ref = pytest.mark.skipif(not HAVE_REF, reason="the original gym-narde is not in the repository: vendor it into "
+                                                    "baseline/_ref (build() with NARDE_REFERENCE_ROOT set, or "
+                                                    "baseline/fetch_ref.py)")
 
 
 def _run(impl, what, n=3):

@@ -90,7 +90,8 @@ def test_obs198_layout_and_bounds():
     assert O.obs198(b, 3, 0, -1)[196:].tolist() == [0, 1]
 
 
-@pytest.mark.skipif(not R.available(), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not R.available(), reason="the original gym-narde is not in the repository: set NARDE_REFERENCE_ROOT "
+                                              "or vendor it with baseline/fetch_ref.py")
 def test_oracle_vs_live_reference_short():
     """Re-runs a short lock-step comparison against the real Python reference (build container only)."""
     import random
