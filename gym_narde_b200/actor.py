@@ -9,8 +9,6 @@ Per lock-step turn, entirely on the GPU and without a host synchronisation:
 """
 from __future__ import annotations
 
-import ctypes as C
-
 from . import _cabi
 
 
@@ -18,7 +16,7 @@ class _SideBatch:
     """Buffers of the second pass over the environments whose legal list exceeds env.max_actions."""
 
     def __init__(self, t, dev, m, cap):
-        self.m, self.cap = m, cap
+        self.cap = cap
         self.lo = t.zeros((m, 16), dtype=t.uint8, device=dev)
         self.hi = t.zeros((m, 16), dtype=t.uint8, device=dev)
         self.dice = t.ones((m, 2), dtype=t.uint8, device=dev)
@@ -67,7 +65,6 @@ class AfterstateActor:
         self.value = t.zeros(n, dtype=t.float32, device=dev)
         self.dice = env.dice                                        # the turn's dice (written by the enumeration)
         self.act_override = t.zeros(n, dtype=t.int64, device=dev)   # chosen actions beyond the stored lists (side batch)
-        self.lib = _cabi.load()
         m = max(256, n // 16) if overflow_slots is None else int(overflow_slots)
         m = -(-m // 128) * 128            # whole tiles of the side batch's kernels
         self.side = None
@@ -78,115 +75,77 @@ class AfterstateActor:
             sb.as_lo = t.zeros((rows, 16), dtype=t.uint8, device=dev)
             sb.as_hi = t.zeros((rows, 16), dtype=t.uint8, device=dev)
             sb.scores = t.zeros(rows, dtype=t.float32, device=dev)
-        self._graph = None
+        self._graph = self._graph_args = None
         self._s2 = t.cuda.Stream(device=dev) if self.side is not None else None
         self._enum_ws = t.zeros(_cabi.workspace_ints(n), dtype=t.int32, device=dev)
-
-    def _stream(self):
-        return C.c_void_p(self.env.torch.cuda.current_stream().cuda_stream)
 
     def afterstates(self, actions, counts):
         """Fill as_lo/as_hi with the afterstates of actions[i, :min(counts[i], cap)]; returns offsets [N]."""
         env = self.env
         # one launch: the device-wide exclusive scan of min(counts, cap) (decoupled look-back), the row count and the
         # rows themselves (narde_afterstates_scan) -- no host-side prefix sum, no torch ops
-        rc = self.lib.narde_afterstates_scan(C.c_void_p(env.lo.data_ptr()), C.c_void_p(env.hi.data_ptr()),
-                                             C.c_void_p(actions.data_ptr()), C.c_void_p(counts.data_ptr()),
-                                             env.num_envs, self.cap, C.c_void_p(self.offsets.data_ptr()),
-                                             C.c_void_p(self.rows_dev.data_ptr()), C.c_void_p(self.as_lo.data_ptr()),
-                                             C.c_void_p(self.as_hi.data_ptr()), None,
-                                             C.c_void_p(self._scan_ws.data_ptr()), 0, None, self._stream())
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_afterstates_scan failed: %d" % rc)
+        _cabi.afterstates_scan(env.lo, env.hi, actions, counts, self.as_lo, self.as_hi, self._scan_ws, offsets=self.offsets,
+                               rows_out=self.rows_dev)
         return self.offsets
 
-    def _side_prepare(self, dice):
+    def _side_prepare(self):
         """Second pass (see __init__): gather -> enumerate with the large capacity -> afterstate rows -> score -> arg-max.  It only
         needs the first pass's enumeration (overflow flags), so it runs on a side stream BESIDE the first pass's rows / scorer /
         arg-max (small latency-bound kernels next to the one-CTA-per-SM scorer); fork / join with stream waits, which a
         CUDA-graph capture records as a branch."""
-        sb, env, P, t = self.side, self.env, C.c_void_p, self.env.torch
+        sb, env, t = self.side, self.env, self.env.torch
         if sb is None:
             return
-        main = t.cuda.current_stream(env.device)
-        self._s2.wait_stream(main)
+        self._s2.wait_stream(t.cuda.current_stream(env.device))
         with t.cuda.stream(self._s2):
-            self._side_prepare_launches(dice)
-
-    def _side_prepare_launches(self, dice):
-        sb, env, P = self.side, self.env, C.c_void_p
-        st = self._stream()
-        rc = self.lib.narde_gather_overflow(P(env.lo.data_ptr()), P(env.hi.data_ptr()), P(dice.data_ptr()),
-                                            P(env.overflow.data_ptr()), env.num_envs, sb.m, P(sb.lo.data_ptr()),
-                                            P(sb.hi.data_ptr()), P(sb.dice.data_ptr()), P(sb.idx.data_ptr()),
-                                            P(sb.ctrl.data_ptr()), st)
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_gather_overflow failed: %d" % rc)
-        _cabi.enumerate_actions_fast(sb.lo, sb.hi, sb.dice, sb.actions, sb.counts, sb.ovf, sb.ws)
-        rc = self.lib.narde_afterstates_scan(P(sb.lo.data_ptr()), P(sb.hi.data_ptr()), P(sb.actions.data_ptr()),
-                                             P(sb.counts.data_ptr()), sb.m, sb.cap, P(sb.offsets.data_ptr()),
-                                             P(sb.rows_dev.data_ptr()), P(sb.as_lo.data_ptr()), P(sb.as_hi.data_ptr()),
-                                             None, P(sb.scan_ws.data_ptr()), sb.rows_cap, P(sb.counts_eff.data_ptr()), st)
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_afterstates_scan failed: %d" % rc)
-        # (the scorer keeps no state between launches, so this one may be queued beside the first pass's: its CTAs get
-        # their SMs when those leave)
-        self.mlp.score_states(sb.as_lo, sb.as_hi, out=sb.scores, rows_dev=sb.rows_dev)
-        rc = self.lib.narde_segment_argmax(P(sb.scores.data_ptr()), P(sb.offsets.data_ptr()), P(sb.counts_eff.data_ptr()),
-                                           P(sb.hi.data_ptr()), sb.m, sb.cap, self.mode, P(sb.choice.data_ptr()),
-                                           P(sb.value.data_ptr()), st)
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_segment_argmax failed: %d" % rc)
+            _cabi.gather_overflow(env.lo, env.hi, self.dice, env.overflow, sb.lo, sb.hi, sb.dice, sb.idx, sb.ctrl)
+            _cabi.enumerate_actions_fast(sb.lo, sb.hi, sb.dice, sb.actions, sb.counts, sb.ovf, sb.ws)
+            _cabi.afterstates_scan(sb.lo, sb.hi, sb.actions, sb.counts, sb.as_lo, sb.as_hi, sb.scan_ws, offsets=sb.offsets,
+                                   rows_out=sb.rows_dev, rows_cap=sb.rows_cap, counts_eff=sb.counts_eff)
+            # (the scorer keeps no state between launches, so this one may be queued beside the first pass's: its CTAs get
+            # their SMs when those leave)
+            self.mlp.score_states(sb.as_lo, sb.as_hi, out=sb.scores, rows_dev=sb.rows_dev)
+            _cabi.segment_argmax(sb.scores, sb.offsets, sb.counts_eff, sb.hi, sb.cap, self.mode, sb.choice, sb.value)
 
     def _side_finish(self):
         """Second pass, after the join: scatter the side batch's choices into self.choice / self.value /
         self.act_override."""
-        sb, env, P, t = self.side, self.env, C.c_void_p, self.env.torch
+        sb, env, t = self.side, self.env, self.env.torch
         if sb is None:
             return
         t.cuda.current_stream(env.device).wait_stream(self._s2)
-        st = self._stream()
-        rc = self.lib.narde_scatter_choice(P(sb.choice.data_ptr()), P(sb.value.data_ptr()), P(sb.idx.data_ptr()),
-                                           P(sb.counts_eff.data_ptr()), P(sb.counts.data_ptr()), sb.m, sb.cap,
-                                           P(self.choice.data_ptr()), P(self.value.data_ptr()), P(sb.ctrl.data_ptr()),
-                                           P(sb.actions.data_ptr()), P(self.act_override.data_ptr()), st)
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_scatter_choice failed: %d" % rc)
+        _cabi.scatter_choice(sb.choice, sb.value, sb.idx, sb.counts_eff, sb.counts, sb.cap, self.choice, self.value, sb.ctrl,
+                             sb.actions, self.act_override)
 
     def uncovered_envs(self):
         """Env turns whose choice was made among the first max_actions actions only (one D2H copy)."""
         return int(self.side.ctrl[2].item()) if self.side is not None else -1
 
+    def _choose_enumerated(self):
+        """The greedy choice once this turn's lists are in env.actions / env.counts / env.overflow and its dice in self.dice:
+        afterstate rows -> score -> arg-max, with the side batch beside them, then its scatter."""
+        env = self.env
+        self._side_prepare()
+        self.afterstates(env.actions, env.counts)
+        self.mlp.score_states(self.as_lo, self.as_hi, out=self.scores, rows_dev=self.rows_dev)
+        _cabi.segment_argmax(self.scores, self.offsets, env.counts, env.hi, self.cap, self.mode, self.choice, self.value)
+        self._side_finish()
+
     def choose(self):
         """roll -> enumerate -> afterstates -> score -> greedy index.  Returns (choice [N] int32, dice [N,2])."""
-        env = self.env
-        env.roll()                        # (writes env.dice, which self.dice is)
-        actions, counts, _ = env.get_valid_actions(self.dice)
-        self._side_prepare(self.dice)
-        self.afterstates(actions, counts)
-        self.mlp.score_states(self.as_lo, self.as_hi, out=self.scores, rows_dev=self.rows_dev)
-        rc = self.lib.narde_segment_argmax(C.c_void_p(self.scores.data_ptr()), C.c_void_p(self.offsets.data_ptr()),
-                                           C.c_void_p(counts.data_ptr()), C.c_void_p(env.hi.data_ptr()), env.num_envs,
-                                           self.cap, self.mode, C.c_void_p(self.choice.data_ptr()),
-                                           C.c_void_p(self.value.data_ptr()), self._stream())
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_segment_argmax failed: %d" % rc)
-        self._side_finish()
+        self.env.roll()                   # (writes env.dice, which self.dice is)
+        self.env.get_valid_actions(self.dice)
+        self._choose_enumerated()
         return self.choice, self.dice
 
     def _play_chosen(self):
         """narde_step_chosen: the lists of this turn are in env.actions / env.counts and the choice is made -- apply it and
         complete the turn (reward, termination, auto-reset, statistics, Box(198)) without enumerating the position again."""
-        env, P = self.env, C.c_void_p
-        flags = (_cabi.REWARD_MOVER12 if env.reward_mode == "mover12" else 0) | (_cabi.AUTORESET if env.autoreset else 0)
-        rc = self.lib.narde_step_chosen(P(env.lo.data_ptr()), P(env.hi.data_ptr()), env.num_envs, env.env_base, env.seed, 0,
-                                        P(self.dice.data_ptr()), P(self.choice.data_ptr()), P(env.actions.data_ptr()), self.cap,
-                                        P(env.counts.data_ptr()), P(self.act_override.data_ptr()), P(env.chosen.data_ptr()),
-                                        P(env.obs.data_ptr()), P(env.reward.data_ptr()), P(env.done.data_ptr()),
-                                        P(env.trunc.data_ptr()), P(env.stats.data_ptr()), flags, env.max_episode_steps,
-                                        P(env._step_dev.data_ptr()), self._stream())
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_step_chosen failed: %d" % rc)
+        env = self.env
+        _cabi.step_chosen(env.lo, env.hi, env.env_base, env.seed, 0, self.dice, self.choice, env.actions, env.counts,
+                          act_override=self.act_override, chosen=env.chosen, obs198=env.obs, reward=env.reward, done=env.done,
+                          truncated=env.trunc, stats=env.stats, flags=env._step_flags(),
+                          max_episode_steps=env.max_episode_steps, step_dev=env._step_dev)
 
     def step(self):
         """One greedy lock-step turn for all envs; returns VecNardeEnv.step's tuple."""
@@ -198,45 +157,37 @@ class AfterstateActor:
         return env.obs, env.reward, env.terminated, env.truncated, env.info
 
     # -- the same turn as ONE CUDA-graph replay ---------------------------------------------------
+    def _enumerate_turn(self):
+        """This turn's legal lists and dice (Philox, step number read from the env's device counter)."""
+        env = self.env
+        _cabi.step_full(env.lo, env.hi, env.env_base, env.seed, 0, actions=env.actions, counts=env.counts,
+                        dice_out=self.dice, done=env.overflow, flags=_cabi.ENUMERATE_ONLY, workspace=self._enum_ws,
+                        step_dev=env._step_dev)
+
     def _enqueue_turn(self):
         """All launches of a greedy turn with the step number read from the env's device counter, so that the
         captured graph can be replayed: enumerate (Philox dice of the turn) -> afterstates -> score -> argmax ->
         fused step with the chosen indices (which re-derives the same dice from the same counter)."""
-        env, t = self.env, self.env.torch
-        flags = (_cabi.REWARD_MOVER12 if env.reward_mode == "mover12" else 0) | (_cabi.AUTORESET if env.autoreset else 0)
-        _cabi.advance_counter(env._step_dev)
-        _cabi.step_full(env.lo, env.hi, env.env_base, env.seed, 0, actions=env.actions, counts=env.counts,
-                        dice_out=self.dice, done=env.overflow, flags=_cabi.ENUMERATE_ONLY, workspace=self._enum_ws,
-                        step_dev=env._step_dev)
-        self._side_prepare(self.dice)
-        self.afterstates(env.actions, env.counts)
-        self.mlp.score_states(self.as_lo, self.as_hi, out=self.scores, rows_dev=self.rows_dev)
-        rc = self.lib.narde_segment_argmax(C.c_void_p(self.scores.data_ptr()), C.c_void_p(self.offsets.data_ptr()),
-                                           C.c_void_p(env.counts.data_ptr()), C.c_void_p(env.hi.data_ptr()), env.num_envs,
-                                           self.cap, self.mode, C.c_void_p(self.choice.data_ptr()),
-                                           C.c_void_p(self.value.data_ptr()), self._stream())
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_segment_argmax failed: %d" % rc)
-        self._side_finish()
+        _cabi.advance_counter(self.env._step_dev)
+        self._enumerate_turn()
+        self._choose_enumerated()
         self._play_chosen()
 
     def step_graph(self):
-        """step() as one CUDA-graph replay (captured on first use; needs the env built with chunks=1)."""
+        """step() as one CUDA-graph replay (captured on first use, and again when env._frozen_args() changed since;
+        needs the env built with chunks=1)."""
         env, t = self.env, self.env.torch
         if len(env._chunks) != 1:
             raise ValueError("step_graph needs an unchunked env")
         env.step_count += 1
-        if self._graph is not None and self._graph_seed != env.seed:
-            self._graph = None           # the seed is a frozen kernel argument of the captured turn
-        if self._graph is None:
+        if self._graph is None or self._graph_args != env._frozen_args():
             self._enqueue_turn_warmup()
             env._step_dev.fill_(env.step_count - 1)
             t.cuda.synchronize(env.device)
             g = t.cuda.CUDAGraph()
             with t.cuda.graph(g):
                 self._enqueue_turn()
-            self._graph = g
-            self._graph_seed = env.seed
+            self._graph, self._graph_args = g, env._frozen_args()
         self._graph.replay()
         return env.obs, env.reward, env.terminated, env.truncated, env.info
 
@@ -245,9 +196,7 @@ class AfterstateActor:
         read-only part of a turn once, outside the graph."""
         env = self.env
         saved = env._step_dev.clone()
-        _cabi.step_full(env.lo, env.hi, env.env_base, env.seed, 0, actions=env.actions, counts=env.counts,
-                        dice_out=self.dice, done=env.overflow, flags=_cabi.ENUMERATE_ONLY, workspace=self._enum_ws,
-                        step_dev=env._step_dev)
+        self._enumerate_turn()
         self.afterstates(env.actions, env.counts)
         self.mlp.score_states(self.as_lo, self.as_hi, out=self.scores, rows_dev=self.rows_dev)
         env._step_dev.copy_(saved)

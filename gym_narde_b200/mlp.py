@@ -9,8 +9,6 @@ weights are re-packed once on the host into the shared-memory operand layout it 
 """
 from __future__ import annotations
 
-import ctypes as C
-
 import numpy as np
 
 from . import _cabi
@@ -64,8 +62,8 @@ class AfterstateMLP:
 
     def __init__(self, w1, b1, w2, b2, w3, b3, w_move2=None, b_move2=None):
         torch = _cabi.require_cuda()
-        lib = _cabi.load()
-        self.torch, self.lib = torch, lib
+        _cabi.load()
+        self.torch = torch
         self._trunk = (w1.cuda(), b1.cuda(), w2.cuda(), b2.cuda())
         self.wpack, self.bias = pack_weights(*self._trunk, w3.cuda(), b3.cuda())
         self.wpack2, _ = pack_weights(*self._trunk, w3.cuda(), b3.cuda(), two_sm=True)
@@ -106,106 +104,49 @@ class AfterstateMLP:
         return cls(w1, sd["feature_network.0.bias"], sd["feature_network.2.weight"], sd["feature_network.2.bias"],
                    sd["move1_head.weight"], sd["move1_head.bias"], *m2)
 
-    def _move1(self, selected_move1, k):
-        t = self.torch
+    def _move1(self, selected_move1):
         if self.wpack_m2 is None:
             raise _cabi.NardeCudaError("move2_head weights were not given (set_move2_head)")
-        m = selected_move1
-        if not (m.is_cuda and m.dim() == 1 and m.shape[0] == k):
-            raise _cabi.NardeCudaError("selected_move1 must be a CUDA tensor [K] of first-move codes")
-        return m.to(t.int32).contiguous()
+        return selected_move1.to(self.torch.int32).contiguous()
 
-    def _stream(self):
-        return C.c_void_p(self.torch.cuda.current_stream().cuda_stream)
-
-    def _check_x(self, x):
+    def _out(self, out, like, *cols):
+        """out, or a new float32 [K, *cols] tensor on like's device (K = len(like))."""
         t = self.torch
-        if not (x.is_cuda and x.dtype == t.float32 and x.is_contiguous() and x.dim() == 2 and x.shape[1] == IN):
-            raise _cabi.NardeCudaError("x must be a contiguous CUDA float32 [K,198] tensor")
-
-    def _check_states(self, lo, hi):
-        t = self.torch
-        for a in (lo, hi):
-            if not (a.is_cuda and a.dtype == t.uint8 and a.is_contiguous() and a.dim() == 2 and a.shape[1] == 16):
-                raise _cabi.NardeCudaError("states must be contiguous CUDA uint8 [K,16] planes")
-        if lo.shape[0] != hi.shape[0]:
-            raise _cabi.NardeCudaError("lo/hi planes differ in length")
-
-    def _run(self, fn, args, what):
-        rc = fn(*args, self._stream())
-        if rc != 0:
-            raise _cabi.NardeCudaError("%s failed: %d" % (what, rc))
+        return t.empty((like.shape[0], *cols), dtype=t.float32, device=like.device) if out is None else out
 
     def forward(self, x, selected_move1=None, out=None):
         """DecomposedDQN.forward (train_deepq_pytorch.py:203-233): move1 Q-values, or, given selected_move1
         (int tensor [K], codes in [0,576)), the move2 Q-values."""
-        t = self.torch
-        self._check_x(x)
-        k = x.shape[0]
-        if out is None:
-            out = t.empty((k, OUT), dtype=t.float32, device=x.device)
+        out = self._out(out, x, OUT)
         if selected_move1 is not None:
-            m = self._move1(selected_move1, k)
-            self._run(self.lib.narde_mlp_forward_move2,
-                      (C.c_void_p(x.data_ptr()), k, C.c_void_p(m.data_ptr()), C.c_void_p(self.wpack_m2.data_ptr()),
-                       C.c_void_p(self.bias_m2.data_ptr()), C.c_void_p(self.w2b_t.data_ptr()), C.c_void_p(out.data_ptr())),
-                      "narde_mlp_forward_move2")
-            return out
-        self._run(self.lib.narde_mlp_forward, (C.c_void_p(x.data_ptr()), k, C.c_void_p(self.wpack.data_ptr()),
-                                               C.c_void_p(self.bias.data_ptr()), C.c_void_p(out.data_ptr())), "narde_mlp_forward")
+            _cabi.mlp_forward_move2(x, self._move1(selected_move1), self.wpack_m2, self.bias_m2, self.w2b_t, out)
+        else:
+            _cabi.mlp_forward(x, self.wpack, self.bias, out)
         return out
 
     def score(self, x, out=None):
-        t = self.torch
-        self._check_x(x)
-        k = x.shape[0]
-        if out is None:
-            out = t.empty(k, dtype=t.float32, device=x.device)
-        self._run(self.lib.narde_mlp_score, (C.c_void_p(x.data_ptr()), k, C.c_void_p(self.wpack.data_ptr()),
-                                             C.c_void_p(self.bias.data_ptr()), C.c_void_p(out.data_ptr())), "narde_mlp_score")
+        out = self._out(out, x)
+        _cabi.mlp_score(x, self.wpack, self.bias, out)
         return out
 
     def forward_states(self, lo, hi, selected_move1=None, out=None):
-        t = self.torch
-        self._check_states(lo, hi)
-        k = lo.shape[0]
-        if out is None:
-            out = t.empty((k, OUT), dtype=t.float32, device=lo.device)
+        out = self._out(out, lo, OUT)
         if selected_move1 is not None:
-            m = self._move1(selected_move1, k)
-            self._run(self.lib.narde_mlp_forward_move2_states,
-                      (C.c_void_p(lo.data_ptr()), C.c_void_p(hi.data_ptr()), k, C.c_void_p(m.data_ptr()),
-                       C.c_void_p(self.wpack_m2.data_ptr()), C.c_void_p(self.bias_m2.data_ptr()),
-                       C.c_void_p(self.w2b_t.data_ptr()), C.c_void_p(out.data_ptr())), "narde_mlp_forward_move2_states")
-            return out
-        self._run(self.lib.narde_mlp_forward_states,
-                  (C.c_void_p(lo.data_ptr()), C.c_void_p(hi.data_ptr()), k, C.c_void_p(self.wpack.data_ptr()),
-                   C.c_void_p(self.bias.data_ptr()), C.c_void_p(out.data_ptr())), "narde_mlp_forward_states")
+            _cabi.mlp_forward_move2_states(lo, hi, self._move1(selected_move1), self.wpack_m2, self.bias_m2, self.w2b_t, out)
+        else:
+            _cabi.mlp_forward_states(lo, hi, self.wpack, self.bias, out)
         return out
 
     def score_states(self, lo, hi, out=None, rows_dev=None):
         """rows_dev: optional int64 CUDA tensor [1]; only min(rows_dev, len(lo)) rows are scored (no host sync)."""
-        t = self.torch
-        self._check_states(lo, hi)
-        k = lo.shape[0]
-        if out is None:
-            out = t.empty(k, dtype=t.float32, device=lo.device)
-        self._run(self.lib.narde_mlp_score_states,
-                  (C.c_void_p(lo.data_ptr()), C.c_void_p(hi.data_ptr()), k,
-                   C.c_void_p(rows_dev.data_ptr() if rows_dev is not None else None), C.c_void_p(self.wpack.data_ptr()),
-                   C.c_void_p(self.bias.data_ptr()), C.c_void_p(out.data_ptr())), "narde_mlp_score_states")
+        out = self._out(out, lo)
+        _cabi.mlp_score_states(lo, hi, self.wpack, self.bias, out, rows_dev)
         return out
 
     def score_states_2sm(self, lo, hi, out=None, rows_dev=None):
         """score_states through the cta_group::2 kernel (clusters of two CTAs, M = 256 per tcgen05.mma)."""
-        t = self.torch
-        self._check_states(lo, hi)
-        k = lo.shape[0]
-        if out is None:
-            out = t.empty(k, dtype=t.float32, device=lo.device)
-        self._run(self.lib.narde_mlp_score_states_2sm, (C.c_void_p(lo.data_ptr()), C.c_void_p(hi.data_ptr()), k,
-                       C.c_void_p(rows_dev.data_ptr() if rows_dev is not None else None), C.c_void_p(self.wpack2.data_ptr()),
-                       C.c_void_p(self.bias.data_ptr()), C.c_void_p(out.data_ptr())), "narde_mlp_score_states_2sm")
+        out = self._out(out, lo)
+        _cabi.mlp_score_states(lo, hi, self.wpack2, self.bias, out, rows_dev, two_sm=True)
         return out
 
     __call__ = forward

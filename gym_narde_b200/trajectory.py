@@ -7,8 +7,6 @@ the ring keeps one 48-byte record per env turn in HBM:
 """
 from __future__ import annotations
 
-import ctypes as C
-
 from . import _cabi
 
 RECORD_BYTES = 48
@@ -22,19 +20,12 @@ class TrajectoryRing:
         self.records = t.zeros((self.capacity, env.num_envs, RECORD_BYTES), dtype=t.uint8, device=env.device)
         self.initial_lo, self.initial_hi = env.lo.clone(), env.hi.clone()   # s_0 (call after env.reset())
         self.cursor = 0          # total turns appended (slot = cursor % capacity)
-        self.lib = _cabi.load()
 
     def append(self):
         """Record the turn VecNardeEnv.step() has just played (one kernel, 48 B per env)."""
-        env, t = self.env, self.env.torch
-        slot = self.records[self.cursor % self.capacity]
-        rc = self.lib.narde_trajectory_append(
-            C.c_void_p(env.lo.data_ptr()), C.c_void_p(env.hi.data_ptr()), C.c_void_p(env.dice.data_ptr()),
-            C.c_void_p(env.chosen.data_ptr()), C.c_void_p(env.reward.data_ptr()), C.c_void_p(env.done.data_ptr()),
-            C.c_void_p(env.trunc.data_ptr()), env.num_envs, C.c_void_p(slot.data_ptr()),
-            C.c_void_p(t.cuda.current_stream().cuda_stream))
-        if rc != 0:
-            raise _cabi.NardeCudaError("narde_trajectory_append failed: %d" % rc)
+        env = self.env
+        _cabi.trajectory_append(env.lo, env.hi, self.records[self.cursor % self.capacity], dice=env.dice, chosen=env.chosen,
+                                reward=env.reward, done=env.done, truncated=env.trunc)
         self.cursor += 1
 
     def step(self, actions=None, dice=None, fraction=False):
@@ -74,8 +65,5 @@ def action_codes(env, actions=None, counts=None):
     counts = env.counts if counts is None else counts
     n, cap = actions.shape
     codes = t.zeros((n, cap, 3), dtype=t.int32, device=actions.device)
-    rc = _cabi.load().narde_action_codes(C.c_void_p(actions.data_ptr()), C.c_void_p(counts.data_ptr()), n, cap,
-                                         C.c_void_p(codes.data_ptr()), C.c_void_p(t.cuda.current_stream().cuda_stream))
-    if rc != 0:
-        raise _cabi.NardeCudaError("narde_action_codes failed: %d" % rc)
+    _cabi.action_codes(actions, counts, codes)
     return codes

@@ -42,7 +42,7 @@ class VecNardeEnv:
         self.write_actions = bool(write_actions)
         self.step_count = 0  # Philox step counter (global, shared by all envs)
         self.use_graph = bool(graph)
-        self._graphs = {}    # (action ptr, dice ptr) -> captured CUDA graph of one step
+        self._graphs = {}    # action-input key -> (captured CUDA graph of one step, the input buffer, _frozen_args())
         n, dev = self.num_envs, self.device
         self.lo = torch.zeros((n, 16), dtype=torch.uint8, device=dev)
         self.hi = torch.zeros((n, 16), dtype=torch.uint8, device=dev)
@@ -87,12 +87,7 @@ class VecNardeEnv:
     def reset(self, *, seed=None, options=None):
         """NardeEnv.reset (narde_env.py:105-120) for every env; returns (obs, {})."""
         if seed is not None:
-            seed = int(seed) & 0xFFFFFFFFFFFFFFFF
-            if seed != self.seed:          # the seed is a frozen kernel argument of every captured step
-                self._graphs.clear()
-                if getattr(self, "_hio", None) is not None:
-                    self._hio_graphs.clear()
-            self.seed = seed
+            self.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
         self.step_count = 0
         self._step_dev.zero_()
         _cabi.reset(self.lo, self.hi, self.env_base, self.seed, 0)
@@ -150,8 +145,7 @@ class VecNardeEnv:
         t = self.torch
         self.step_count += 1
         if self.rules == "full":
-            flags = (_cabi.REWARD_MOVER12 if self.reward_mode == "mover12" else 0) | (
-                _cabi.AUTORESET if self.autoreset else 0) | (_cabi.ACTION_FRACTION if fraction and actions is not None else 0)
+            flags = self._step_flags(fraction=fraction and actions is not None)
             # A captured graph freezes the kernel arguments, so graphs are cached per action-input buffer
             # (identified by its device pointer; the tensor is kept alive by the cache) and replayed when the
             # same persistent buffer is passed again.  Up to 8 buffers are cached; anything else (fresh
@@ -166,9 +160,8 @@ class VecNardeEnv:
                         key = None
             if key is not None:
                 ent = self._graphs.get(key)
-                if ent is None:
-                    ent = (self._capture(actions, dice, flags), actions)
-                    self._graphs[key] = ent
+                if ent is None or ent[2] != self._frozen_args():
+                    ent = self._graphs[key] = (self._capture(actions, dice, flags), actions, self._frozen_args())
                 ent[0].replay()
             else:
                 self._step_dev.fill_(self.step_count)
@@ -182,6 +175,17 @@ class VecNardeEnv:
             _cabi.step_ref(self.lo, self.hi, dice, actions, self.obs, self.reward, self.done,
                            max_episode_steps=self.max_episode_steps, truncated=self.trunc)
         return self.obs, self.reward, self.terminated, self.truncated, self.info
+
+    def _step_flags(self, fraction=False, packed=False):
+        """The flags word of this env's full-rules step launches."""
+        return ((_cabi.REWARD_MOVER12 if self.reward_mode == "mover12" else 0) | (_cabi.AUTORESET if self.autoreset else 0)
+                | (_cabi.ACTION_FRACTION if fraction else 0) | (_cabi.PACK_RESULT if packed else 0))
+
+    def _frozen_args(self):
+        """The kernel arguments a captured CUDA graph freezes that reset(seed=...) and load_state_dict() can change.  Every
+        holder of a captured graph (this env's step caches, HostPipeline, AfterstateActor) records this value at capture
+        and captures again when it differs before a replay."""
+        return self.seed, self.env_base
 
     def _launch_full(self, actions, dice, flags, dev_advance=False):
         """Enqueue one fused step: every chunk on its own stream (fork/join around the current stream).
@@ -271,9 +275,7 @@ class VecNardeEnv:
             raise ValueError("step_host needs rules='full'")
         io = self.host_io()
         self.step_count += 1
-        flags = (_cabi.REWARD_MOVER12 if self.reward_mode == "mover12" else 0) | (
-            _cabi.AUTORESET if self.autoreset else 0) | (_cabi.ACTION_FRACTION if fraction else 0) | (
-            _cabi.PACK_RESULT if packed else 0)
+        flags = self._step_flags(fraction, packed)
         src = io["actions"] if actions is None else actions
         if not (src.is_pinned() and src.dtype == t.int32 and src.is_contiguous() and src.numel() == self.num_envs):
             raise _cabi.NardeCudaError("step_host actions must be a pinned contiguous int32 [N] host tensor")
@@ -284,10 +286,9 @@ class VecNardeEnv:
             raise _cabi.NardeCudaError("step_host needs an unchunked env (chunks=1)")
         key = (src.data_ptr(), bool(fraction), bool(packed), bool(dma_in), obs)
         ent = self._hio_graphs.get(key)
-        g = ent[0] if ent is not None else None
-        if g is None and len(self._hio_graphs) >= 32:
+        if ent is None and len(self._hio_graphs) >= 32:
             raise _cabi.NardeCudaError("step_host: more than 32 distinct host action buffers")
-        if g is None:
+        if ent is None or ent[2] != self._frozen_args():
             self._step_dev.fill_(self.step_count - 1)
             t.cuda.synchronize(self.device)
             g = t.cuda.CUDAGraph()
@@ -311,8 +312,8 @@ class VecNardeEnv:
                                 workspace=self._ws_adv if adv else self._workspaces[0], step_dev=self._step_dev,
                                 mirror_lo=io["lo"] if obs == "packed" else (io["rec"] if compact else None),
                                 mirror_hi=io["hi"] if obs == "packed" else None)
-            self._hio_graphs[key] = (g, src)
-        g.replay()
+            ent = self._hio_graphs[key] = (g, src, self._frozen_args())
+        ent[0].replay()
         return io
 
     def host_pipeline(self, depth=8, fraction=False):
@@ -336,9 +337,6 @@ class VecNardeEnv:
         self.hi.copy_(sd["hi"])
         self.seed, self.step_count, self.env_base = sd["seed"], sd["step_count"], sd["env_base"]
         self._step_dev.fill_(self.step_count)
-        self._graphs.clear()  # the seed is a frozen kernel argument
-        if getattr(self, "_hio", None) is not None:
-            self._hio_graphs.clear()
 
     def close(self):
         pass
@@ -366,12 +364,11 @@ class HostPipeline:
         self.truncated = t.zeros((depth, n), dtype=t.uint8).pin_memory()
         self._d_act = [t.zeros(n, dtype=t.int32, device=dev) for _ in range(2)]
         self._s_in = t.cuda.Stream(device=dev)
-        self._graph = None
+        self._graph = self._graph_args = None
 
     def _capture(self):
         env, t, D = self.env, self.env.torch, self.depth
-        flags = (_cabi.REWARD_MOVER12 if env.reward_mode == "mover12" else 0) | (
-            _cabi.AUTORESET if env.autoreset else 0) | (_cabi.ACTION_FRACTION if self.fraction else 0)
+        flags = env._step_flags(self.fraction)
         env._step_dev.fill_(env.step_count)
         t.cuda.synchronize(env.device)
         g = t.cuda.CUDAGraph()
@@ -403,10 +400,7 @@ class HostPipeline:
 
     def run(self):
         """Play the next `depth` turns (one graph replay)."""
-        if self._graph is not None and self._graph_seed != self.env.seed:
-            self._graph = None               # the seed is a frozen kernel argument of the captured turns
-        if self._graph is None:
-            self._graph = self._capture()
-            self._graph_seed = self.env.seed
+        if self._graph is None or self._graph_args != self.env._frozen_args():
+            self._graph, self._graph_args = self._capture(), self.env._frozen_args()
         self._graph.replay()
         self.env.step_count += self.depth

@@ -78,6 +78,51 @@ def test_no_cpu_fallback():
         _cabi.reset(torch.zeros((1, 16), dtype=torch.uint8), torch.zeros((1, 16), dtype=torch.uint8), 0, 0, 0)
 
 
+def test_actor_trajectory_and_mlp_wrappers_have_no_cpu_fallback():
+    """Every C-ABI wrapper of the actor, trajectory and MLP entry points raises NardeCudaError for CPU tensors (with or
+    without a CUDA device present)."""
+    import torch
+    u8, i16, i32, i64, f32 = torch.uint8, torch.int16, torch.int32, torch.int64, torch.float32
+    z = lambda dt, *shape: torch.zeros(shape, dtype=dt)
+    n, cap, m = 4, 8, 32
+    lo, hi, acts, counts = z(u8, n, 16), z(u8, n, 16), z(i64, n, cap), z(i32, n)
+    x, wpack, bias, w2b_t, move1 = z(f32, n, 198), z(i16, 64), z(f32, 1088), z(f32, 576, 576), z(i32, n)
+    calls = [
+        ("afterstates", (lo, hi, acts, counts, z(i64, n), z(u8, n * cap, 16), z(u8, n * cap, 16))),
+        ("afterstates_scan", (lo, hi, acts, counts, z(u8, n * cap, 16), z(u8, n * cap, 16), z(i64, 5))),
+        ("gather_overflow", (lo, hi, z(u8, n, 2), z(u8, n), z(u8, m, 16), z(u8, m, 16), z(u8, m, 2), z(i32, m), z(i32, 4))),
+        ("scatter_choice", (z(i32, m), z(f32, m), z(i32, m), z(i32, m), z(i32, m), cap, z(i32, n), z(f32, n), z(i32, 4))),
+        ("segment_argmax", (z(f32, n * cap), z(i64, n), counts, hi, cap, 0, z(i32, n))),
+        ("step_chosen", (lo, hi, 0, 0, 0, z(u8, n, 2), z(i32, n), acts, counts)),
+        ("action_codes", (acts, counts, z(i32, n, cap, 3))),
+        ("trajectory_append", (lo, hi, z(u8, n, 48))),
+        ("mlp_forward", (x, wpack, bias, z(f32, n, 576))),
+        ("mlp_score", (x, wpack, bias, z(f32, n))),
+        ("mlp_forward_states", (lo, hi, wpack, bias, z(f32, n, 576))),
+        ("mlp_score_states", (lo, hi, wpack, bias, z(f32, n))),
+        ("mlp_score_states", (lo, hi, wpack, bias, z(f32, n), None, True)),
+        ("mlp_forward_move2", (x, move1, wpack, bias, w2b_t, z(f32, n, 576))),
+        ("mlp_forward_move2_states", (lo, hi, move1, wpack, bias, w2b_t, z(f32, n, 576))),
+    ]
+    for name, args in calls:
+        with pytest.raises(_cabi.NardeCudaError):
+            getattr(_cabi, name)(*args)
+
+
+def test_only_cabi_calls_the_library():
+    """_cabi.py is the package's one bridge to the C ABI: no other module builds ctypes pointers or calls a narde_*
+    symbol itself.  (envs/, the single-env facade, keeps pointers cached at construction: its per-call latency is its
+    point.)"""
+    pkg = os.path.join(ROOT, "gym_narde_b200")
+    for dp, _, files in os.walk(pkg):
+        if os.path.relpath(dp, pkg).split(os.sep)[0] == "envs":
+            continue
+        for f in files:
+            if f.endswith(".py") and f != "_cabi.py":
+                src = open(os.path.join(dp, f)).read()
+                assert "c_void_p" not in src and not re.search(r"\.narde_\w+\s*\(", src), (dp, f)
+
+
 def test_product_never_imports_the_oracle():
     pkg = os.path.join(ROOT, "gym_narde_b200")
     for dp, _, files in os.walk(pkg):

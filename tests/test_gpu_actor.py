@@ -126,8 +126,7 @@ def test_afterstates_scan_equals_host_prefix_sum_version():
         ref_lo = torch.zeros((K + 1, 16), dtype=torch.uint8, device="cuda")
         ref_hi = torch.zeros_like(ref_lo)
         ref_env = torch.full((K + 1,), -1, dtype=torch.int32, device="cuda")
-        assert lib.narde_afterstates(P(env.lo), P(env.hi), P(acts), P(counts), P(off_ref), n, cap, P(ref_lo), P(ref_hi),
-                                     P(ref_env), st) == 0
+        _cabi.afterstates(env.lo, env.hi, acts, counts, off_ref, ref_lo, ref_hi, ref_env)
         for rep in range(2):           # the scratch words are left ready for the next call
             lo2, hi2 = torch.zeros_like(ref_lo), torch.zeros_like(ref_hi)
             env2 = torch.full_like(ref_env, -1)
@@ -144,13 +143,10 @@ def test_actor_scores_every_legal_action_beyond_the_stored_capacity():
     """ADVICE r1: the greedy choice must look at EVERY legal action (DQNAgent.act, train_deepq_pytorch.py:430-507), not
     at the first env.max_actions.  With a tiny stored capacity most envs overflow; the actor's choice (main pass +
     side-batch pass) must equal the arg-max over the complete list enumerated with a capacity that holds everything."""
-    import ctypes as C
     import torch
     from gym_narde_b200 import VecNardeEnv, AfterstateMLP, AfterstateActor, _cabi
     fn, head = _net()
     mlp = AfterstateMLP.from_module(fn, head)
-    lib = _cabi.load()
-    P = lambda t: C.c_void_p(t.data_ptr())
     n, cap, big = 1536, 8, 2048
     for mode in ("max", "white_value"):
         env = VecNardeEnv(n, seed=31, max_actions=cap)
@@ -170,8 +166,7 @@ def test_actor_scores_every_legal_action_beyond_the_stored_capacity():
             K = int(c.sum().item())
             lo2 = torch.zeros((K + 1, 16), dtype=torch.uint8, device="cuda")
             hi2 = torch.zeros_like(lo2)
-            st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-            assert lib.narde_afterstates(P(env.lo), P(env.hi), P(acts_b), P(cnt_b), P(off), n, big, P(lo2), P(hi2), None, st) == 0
+            _cabi.afterstates(env.lo, env.hi, acts_b, cnt_b, off, lo2, hi2)
             sc = mlp.score_states(lo2[:K].contiguous(), hi2[:K].contiguous())
             dense = torch.full((n, int(c.max().item()) + 1), float("-inf"), device="cuda")
             col = torch.arange(dense.shape[1], device="cuda")[None, :]
@@ -227,3 +222,92 @@ def test_step_chosen_equals_fused_step_with_the_same_choice():
         if cap == 6:
             assert beyond > 1000          # actions that were never stored in the main batch's lists were played
         assert int(actor.act_override.abs().sum().item()) == 0   # every override was consumed
+
+
+def test_short_or_mistyped_buffers_are_refused_before_any_launch():
+    """A short `out`, an int32 rows_dev and a short afterstate buffer raise NardeCudaError, and nothing is launched: the
+    outputs keep their sentinel values."""
+    import torch
+    from gym_narde_b200 import VecNardeEnv, AfterstateMLP, _cabi
+    fn, head = _net()
+    mlp = AfterstateMLP.from_module(fn, head)
+    n, cap = 512, 16
+    env = VecNardeEnv(n, seed=3, max_actions=cap)
+    env.reset()
+    acts, counts, _ = env.get_valid_actions()
+    torch.cuda.synchronize()
+    score = torch.full((n - 1,), 7.0, device="cuda")
+    q = torch.full((n, 575), 7.0, device="cuda")
+    score_full = torch.full((n,), 7.0, device="cuda")
+    rows = torch.full((1,), -5, dtype=torch.int64, device="cuda")
+    with pytest.raises(_cabi.NardeCudaError, match="out must have shape"):
+        mlp.score_states(env.lo, env.hi, out=score)
+    with pytest.raises(_cabi.NardeCudaError, match="out must have shape"):
+        mlp.forward_states(env.lo, env.hi, out=q)
+    with pytest.raises(_cabi.NardeCudaError, match="out must have shape"):
+        mlp.forward(env.obs, out=score_full)                      # q rows are [K,576], not [K]
+    with pytest.raises(_cabi.NardeCudaError, match="rows_dev must have dtype"):
+        mlp.score_states(env.lo, env.hi, out=score_full, rows_dev=torch.full((1,), n, dtype=torch.int32, device="cuda"))
+    scratch = torch.zeros(n // 128 + 4, dtype=torch.int64, device="cuda")
+    short = [torch.zeros((n * cap - 1, 16), dtype=torch.uint8, device="cuda") for _ in range(2)]
+    with pytest.raises(_cabi.NardeCudaError, match="as_lo must have at least"):
+        _cabi.afterstates_scan(env.lo, env.hi, acts, counts, *short, scratch, rows_out=rows)     # rows_cap 0: n * cap rows
+    with pytest.raises(_cabi.NardeCudaError, match="as_lo must have at least"):
+        _cabi.afterstates_scan(env.lo, env.hi, acts, counts, *short, scratch, rows_out=rows, rows_cap=n * cap)
+    torch.cuda.synchronize()
+    assert (score == 7).all() and (q == 7).all() and (score_full == 7).all()
+    assert int(rows.item()) == -5 and int(scratch.abs().sum().item()) == 0
+
+
+def test_captured_graphs_follow_a_loaded_env_base():
+    """env_base is a frozen kernel argument of every captured graph, like the seed: after load_state_dict() of a state
+    with another env_base (same seed), the replays of AfterstateActor.step_graph(), HostPipeline.run() and the env's own
+    step graph play the turns of a freshly built env given the same state."""
+    import torch
+    from gym_narde_b200 import VecNardeEnv, AfterstateMLP, AfterstateActor
+    fn, head = _net()
+    mlp = AfterstateMLP.from_module(fn, head)
+    n, cap, depth = 2048, 64, 4
+    src = VecNardeEnv(n, seed=11, max_actions=cap, env_base=5 * n)
+    src.reset()
+    for _ in range(20):
+        src.step()
+    sd = src.state_dict()
+
+    def fresh():
+        e = VecNardeEnv(n, seed=99, max_actions=cap)
+        e.load_state_dict(sd)
+        return e
+
+    a = VecNardeEnv(n, seed=11, max_actions=cap)
+    actor = AfterstateActor(a, mlp)
+    a.reset()
+    for _ in range(3):
+        actor.step_graph()                  # captured with env_base 0
+    a.load_state_dict(sd)
+    b = fresh()
+    actor_b = AfterstateActor(b, mlp)
+    for t in range(3):
+        actor.step_graph()
+        actor_b.step()
+        assert torch.equal(a.lo, b.lo) and torch.equal(a.hi, b.hi) and torch.equal(a.chosen, b.chosen), t
+
+    a = VecNardeEnv(n, seed=11, max_actions=cap)
+    a.reset()
+    pipe = a.host_pipeline(depth=depth)
+    pipe.run()
+    a.step()                                # the env's own graph of a Philox-random step
+    a.load_state_dict(sd)
+    b = fresh()
+    acts = torch.randint(0, 12, (depth, n), generator=torch.Generator().manual_seed(2), dtype=torch.int32)
+    pipe.actions.copy_(acts)
+    pipe.run()
+    want_r = []
+    for k in range(depth):
+        b.step(acts[k].cuda())
+        want_r.append(b.reward.cpu())
+    torch.cuda.synchronize()
+    assert torch.equal(a.lo, b.lo) and torch.equal(a.hi, b.hi) and torch.equal(pipe.reward, torch.stack(want_r))
+    a.step()
+    b.step()
+    assert torch.equal(a.lo, b.lo) and torch.equal(a.hi, b.hi) and torch.equal(a.dice, b.dice)
