@@ -66,10 +66,12 @@ _SIGNATURES = {
     "narde_afterstates": ([_vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp], _int),
     "narde_afterstates_scan": ([_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp], _int),
     "narde_gather_overflow": ([_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp], _int),
+    "narde_gather_overflow_clear": ([_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _int),
     "narde_scatter_choice": ([_vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp], _int),
     "narde_step_chosen": ([_vp, _vp, _i64, _i64, _u64, _u64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                            _i32, _i32, _vp, _vp], _int),
     "narde_segment_argmax": ([_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp], _int),
+    "narde_segment_sample": ([_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _i64, _u64, _u64, _vp, _vp, _vp, _vp, _vp], _int),
     "narde_obs198": ([_vp, _vp, _i64, _vp, _vp], _int),
     "narde_obs24": ([_vp, _vp, _i64, _vp, _vp], _int),
     "narde_apply_actions": ([_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp], _int),
@@ -349,18 +351,20 @@ def afterstates_scan(lo, hi, actions, counts, as_lo, as_hi, scratch, offsets=Non
     _check(rc, "narde_afterstates_scan")
 
 
-def gather_overflow(lo, hi, dice, overflow, sub_lo, sub_hi, sub_dice, sub_idx, ctrl):
+def gather_overflow(lo, hi, dice, overflow, sub_lo, sub_hi, sub_dice, sub_idx, ctrl, act_override=None):
+    """act_override ([n] int64, optional) is zeroed for every env: the turn starts with no stale override."""
     import torch
 
     dev, n, m = _device(), lo.shape[0], sub_lo.shape[0]
     if m % 32:
         raise NardeCudaError("the side batch must have a multiple of 32 slots, got %d" % m)
-    rc = load().narde_gather_overflow(
+    rc = load().narde_gather_overflow_clear(
         _ptr(lo, torch.uint8, "lo", dev, (n, 16)), _ptr(hi, torch.uint8, "hi", dev, (n, 16)),
         _ptr(dice, torch.uint8, "dice", dev, (n, 2)), _ptr(overflow, torch.uint8, "overflow", dev, (n,)), n, m,
         _ptr(sub_lo, torch.uint8, "sub_lo", dev, (m, 16)), _ptr(sub_hi, torch.uint8, "sub_hi", dev, (m, 16)),
         _ptr(sub_dice, torch.uint8, "sub_dice", dev, (m, 2)), _ptr(sub_idx, torch.int32, "sub_idx", dev, (m,)),
-        _ptr(ctrl, torch.int32, "ctrl", dev, (_ANY,), 4), _stream())
+        _ptr(ctrl, torch.int32, "ctrl", dev, (_ANY,), 4), _ptr(act_override, torch.int64, "act_override", dev, (n,)),
+        _stream())
     _check(rc, "narde_gather_overflow")
 
 
@@ -389,6 +393,23 @@ def segment_argmax(score, offsets, counts, hi, cap, mode, idx_out, best_out=None
         _ptr(counts, torch.int32, "counts", dev, (n,)), _ptr(hi, torch.uint8, "hi", dev, (n, 16)), n, cap, mode,
         _ptr(idx_out, torch.int32, "idx_out", dev, (n,)), _ptr(best_out, torch.float32, "best_out", dev, (n,)), _stream())
     _check(rc, "narde_segment_argmax")
+
+
+def segment_sample(score, offsets, counts, hi, cap, mode, env_base, seed, step, params, idx_out, value_out=None,
+                   env_idx=None, step_dev=None):
+    """narde_segment_sample: segment_argmax with epsilon-greedy / softmax exploration, params = float32 [2] on the device
+    {epsilon, 1 / temperature}; env_idx ([n] int32, optional) maps slot i to its env (env_base + env_idx[i]); step_dev
+    (int64 [1], optional) overrides `step` with the device-resident turn number."""
+    import torch
+
+    dev, n = _device(), hi.shape[0]
+    rc = load().narde_segment_sample(
+        _ptr(score, torch.float32, "score", dev, (_ANY,)), _ptr(offsets, torch.int64, "offsets", dev, (n,)),
+        _ptr(counts, torch.int32, "counts", dev, (n,)), _ptr(hi, torch.uint8, "hi", dev, (n, 16)), n, cap, mode,
+        _ptr(env_idx, torch.int32, "env_idx", dev, (n,)), env_base, seed & 0xFFFFFFFFFFFFFFFF, step,
+        _ptr(step_dev, torch.int64, "step_dev", dev, (1,)), _ptr(params, torch.float32, "params", dev, (2,)),
+        _ptr(idx_out, torch.int32, "idx_out", dev, (n,)), _ptr(value_out, torch.float32, "value_out", dev, (n,)), _stream())
+    _check(rc, "narde_segment_sample")
 
 
 def step_chosen(lo, hi, env_base, seed, step, dice, choice, actions, counts, act_override=None, chosen=None, obs198=None,

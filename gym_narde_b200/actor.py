@@ -1,15 +1,19 @@
-"""Batched afterstate-greedy actor (SURVEY.md section 8(f) rank 1): the device-resident replacement of
-the per-move loop of DQNAgent.act (train_deepq_pytorch.py:411-600).
+"""Batched afterstate actor (SURVEY.md section 8(f) rank 1): the device-resident replacement of
+the per-move loop of DQNAgent.act (train_deepq_pytorch.py:411-600), greedy or exploring.
 
 Per lock-step turn, entirely on the GPU and without a host synchronisation:
     roll (Philox) -> get_valid_actions (full legal-turn enumeration) -> afterstate of every legal
     action (narde_afterstates) -> Box(198) encoding + DecomposedDQN(198) forward + max_a Q on the
-    tcgen05 tensor cores (narde_mlp_score_states) -> greedy choice per env (narde_segment_argmax)
-    -> VecNardeEnv.step(action_idx, dice).
+    tcgen05 tensor cores (narde_mlp_score_states) -> greedy choice per env (narde_segment_argmax), or
+    epsilon-greedy / softmax once exploration is on (narde_segment_sample) -> VecNardeEnv.step(action_idx, dice).
 """
 from __future__ import annotations
 
+import math
+
 from . import _cabi
+
+_FLT_MAX = 3.4028234663852886e38
 
 
 class _SideBatch:
@@ -35,9 +39,18 @@ class _SideBatch:
 
 
 class AfterstateActor:
-    def __init__(self, env, mlp, mode="max", overflow_slots=None, overflow_cap=3072, overflow_rows=None):
+    def __init__(self, env, mlp, mode="max", overflow_slots=None, overflow_cap=3072, overflow_rows=None, epsilon=0.0,
+                 temperature=0.0):
         """env: VecNardeEnv(rules="full"); mlp: AfterstateMLP; mode: "max" (the mover maximises the score)
         or "white_value" (the net scores positions for WHITE: WHITE maximises, BLACK minimises).
+
+        Exploration (DQNAgent.act's epsilon, decayed by the trainer; see set_exploration): each env turn explores with
+        probability `epsilon` and then plays the env's own uniform random action (the one VecNardeEnv.step() plays
+        without actions: epsilon=1 is exactly that policy); otherwise, with `temperature` > 0, it samples
+        softmax(score / temperature) (the score negated for BLACK in "white_value" mode), else it plays the arg-max.
+        The random words come from the env's Philox stream keyed by seed, global env id and turn number
+        (include/narde_b200.h, narde_segment_sample): results do not depend on sharding and can be recomputed on the host.
+        `value` holds the score of the action chosen.
 
         Every legal action is scored, as DQNAgent.act does (train_deepq_pytorch.py:430-507): environments whose list
         is longer than env.max_actions (doubles turns, up to ~1300 actions; 0.5-1 % of the envs in self-play) get a
@@ -76,8 +89,32 @@ class AfterstateActor:
             sb.as_hi = t.zeros((rows, 16), dtype=t.uint8, device=dev)
             sb.scores = t.zeros(rows, dtype=t.float32, device=dev)
         self._graph = self._graph_args = None
+        self._params = t.zeros(2, dtype=t.float32, device=dev)   # {epsilon, 1 / temperature}, read by the kernels
+        self._sampling = False        # narde_segment_sample from the first time exploration is switched on
+        self.epsilon = self.temperature = 0.0
+        self.set_exploration(epsilon, temperature)
         self._s2 = t.cuda.Stream(device=dev) if self.side is not None else None
         self._enum_ws = t.zeros(_cabi.workspace_ints(n), dtype=t.int32, device=dev)
+
+    def set_exploration(self, epsilon=None, temperature=None):
+        """Set the exploration rate epsilon in [0, 1] and the softmax temperature (>= 0; 0 = arg-max) for the next
+        turns; None keeps the current value.  The values live in device memory: changing them (e.g. decaying epsilon
+        every episode) never recaptures step_graph()'s CUDA graph.  Only the first switch from greedy to exploring does,
+        once."""
+        eps = self.epsilon if epsilon is None else float(epsilon)
+        tau = self.temperature if temperature is None else float(temperature)
+        if not 0.0 <= eps <= 1.0:
+            raise ValueError("epsilon must be in [0, 1], got %r" % (epsilon,))
+        if not (math.isfinite(tau) and tau >= 0.0):
+            raise ValueError("temperature must be finite and >= 0, got %r" % (temperature,))
+        inv_tau = 1.0 / tau if tau > 0.0 else 0.0
+        if inv_tau > _FLT_MAX:
+            raise ValueError("temperature %r is too small: 1 / temperature overflows float32" % (temperature,))
+        self.epsilon, self.temperature = eps, tau
+        # (a stream-ordered copy: turns enqueued before it keep the old values, later ones see the new)
+        self._params.copy_(self.env.torch.tensor([eps, inv_tau], dtype=self.env.torch.float32))
+        if eps > 0.0 or tau > 0.0:
+            self._sampling = True
 
     def afterstates(self, actions, counts):
         """Fill as_lo/as_hi with the afterstates of actions[i, :min(counts[i], cap)]; returns offsets [N]."""
@@ -88,8 +125,18 @@ class AfterstateActor:
                                rows_out=self.rows_dev)
         return self.offsets
 
-    def _side_prepare(self):
-        """Second pass (see __init__): gather -> enumerate with the large capacity -> afterstate rows -> score -> arg-max.  It only
+    def _segment_choice(self, score, offsets, counts, hi, cap, choice, value, step, step_dev, env_idx=None):
+        """The choice per env over its scores: narde_segment_argmax until exploration was first switched on, then
+        narde_segment_sample (bit-equal to it with zero parameters)."""
+        if not self._sampling:
+            _cabi.segment_argmax(score, offsets, counts, hi, cap, self.mode, choice, value)
+            return
+        env = self.env
+        _cabi.segment_sample(score, offsets, counts, hi, cap, self.mode, env.env_base, env.seed, step, self._params, choice,
+                             value, env_idx=env_idx, step_dev=step_dev)
+
+    def _side_prepare(self, step, step_dev):
+        """Second pass (see __init__): gather -> enumerate with the large capacity -> afterstate rows -> score -> choice.  It only
         needs the first pass's enumeration (overflow flags), so it runs on a side stream BESIDE the first pass's rows / scorer /
         arg-max (small latency-bound kernels next to the one-CTA-per-SM scorer); fork / join with stream waits, which a
         CUDA-graph capture records as a branch."""
@@ -98,14 +145,17 @@ class AfterstateActor:
             return
         self._s2.wait_stream(t.cuda.current_stream(env.device))
         with t.cuda.stream(self._s2):
-            _cabi.gather_overflow(env.lo, env.hi, self.dice, env.overflow, sb.lo, sb.hi, sb.dice, sb.idx, sb.ctrl)
+            _cabi.gather_overflow(env.lo, env.hi, self.dice, env.overflow, sb.lo, sb.hi, sb.dice, sb.idx, sb.ctrl,
+                                  act_override=self.act_override)
             _cabi.enumerate_actions_fast(sb.lo, sb.hi, sb.dice, sb.actions, sb.counts, sb.ovf, sb.ws)
             _cabi.afterstates_scan(sb.lo, sb.hi, sb.actions, sb.counts, sb.as_lo, sb.as_hi, sb.scan_ws, offsets=sb.offsets,
                                    rows_out=sb.rows_dev, rows_cap=sb.rows_cap, counts_eff=sb.counts_eff)
             # (the scorer keeps no state between launches, so this one may be queued beside the first pass's: its CTAs get
             # their SMs when those leave)
             self.mlp.score_states(sb.as_lo, sb.as_hi, out=sb.scores, rows_dev=sb.rows_dev)
-            _cabi.segment_argmax(sb.scores, sb.offsets, sb.counts_eff, sb.hi, sb.cap, self.mode, sb.choice, sb.value)
+            # (the same rule over the whole list: the same coin and, per action index, the same noise as the first pass)
+            self._segment_choice(sb.scores, sb.offsets, sb.counts_eff, sb.hi, sb.cap, sb.choice, sb.value, step, step_dev,
+                                 env_idx=sb.idx)
 
     def _side_finish(self):
         """Second pass, after the join: scatter the side batch's choices into self.choice / self.value /
@@ -121,21 +171,23 @@ class AfterstateActor:
         """Env turns whose choice was made among the first max_actions actions only (one D2H copy)."""
         return int(self.side.ctrl[2].item()) if self.side is not None else -1
 
-    def _choose_enumerated(self):
-        """The greedy choice once this turn's lists are in env.actions / env.counts / env.overflow and its dice in self.dice:
-        afterstate rows -> score -> arg-max, with the side batch beside them, then its scatter."""
+    def _choose_enumerated(self, step, step_dev=None):
+        """The choice once this turn's lists are in env.actions / env.counts / env.overflow and its dice in self.dice:
+        afterstate rows -> score -> arg-max (or sample), with the side batch beside them, then its scatter.  step / step_dev:
+        the turn number the dice were rolled with, which keys the exploration's random words."""
         env = self.env
-        self._side_prepare()
+        self._side_prepare(step, step_dev)
         self.afterstates(env.actions, env.counts)
         self.mlp.score_states(self.as_lo, self.as_hi, out=self.scores, rows_dev=self.rows_dev)
-        _cabi.segment_argmax(self.scores, self.offsets, env.counts, env.hi, self.cap, self.mode, self.choice, self.value)
+        self._segment_choice(self.scores, self.offsets, env.counts, env.hi, self.cap, self.choice, self.value, step, step_dev)
         self._side_finish()
 
     def choose(self):
-        """roll -> enumerate -> afterstates -> score -> greedy index.  Returns (choice [N] int32, dice [N,2])."""
+        """roll -> enumerate -> afterstates -> score -> greedy (or exploring) index.  Returns (choice [N] int32, dice [N,2]).
+        The choice may be played by VecNardeEnv.step(choice, dice) as well as by step()."""
         self.env.roll()                   # (writes env.dice, which self.dice is)
         self.env.get_valid_actions(self.dice)
-        self._choose_enumerated()
+        self._choose_enumerated(self.env.step_count + 1)      # the turn number env.roll() used
         return self.choice, self.dice
 
     def _play_chosen(self):
@@ -148,7 +200,7 @@ class AfterstateActor:
                           max_episode_steps=env.max_episode_steps, step_dev=env._step_dev)
 
     def step(self):
-        """One greedy lock-step turn for all envs; returns VecNardeEnv.step's tuple."""
+        """One lock-step turn for all envs; returns VecNardeEnv.step's tuple."""
         env = self.env
         self.choose()
         env.step_count += 1
@@ -170,24 +222,25 @@ class AfterstateActor:
         fused step with the chosen indices (which re-derives the same dice from the same counter)."""
         _cabi.advance_counter(self.env._step_dev)
         self._enumerate_turn()
-        self._choose_enumerated()
+        self._choose_enumerated(0, step_dev=self.env._step_dev)
         self._play_chosen()
 
     def step_graph(self):
-        """step() as one CUDA-graph replay (captured on first use, and again when env._frozen_args() changed since;
-        needs the env built with chunks=1)."""
+        """step() as one CUDA-graph replay (captured on first use, and again when env._frozen_args() or the greedy /
+        exploring switch changed since; needs the env built with chunks=1)."""
         env, t = self.env, self.env.torch
         if len(env._chunks) != 1:
             raise ValueError("step_graph needs an unchunked env")
         env.step_count += 1
-        if self._graph is None or self._graph_args != env._frozen_args():
+        key = (env._frozen_args(), self._sampling)
+        if self._graph is None or self._graph_args != key:
             self._enqueue_turn_warmup()
             env._step_dev.fill_(env.step_count - 1)
             t.cuda.synchronize(env.device)
             g = t.cuda.CUDAGraph()
             with t.cuda.graph(g):
                 self._enqueue_turn()
-            self._graph, self._graph_args = g, env._frozen_args()
+            self._graph, self._graph_args = g, key
         self._graph.replay()
         return env.obs, env.reward, env.terminated, env.truncated, env.info
 

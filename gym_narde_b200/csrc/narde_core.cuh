@@ -948,6 +948,10 @@ NHD int die_from_word(uint32_t w) { return 1 + (int)mulhi32(w, 6u); }
 NHD U4 turn_random(uint64_t seed, uint32_t env, uint64_t step) {
   return philox4x32_10(env, (uint32_t)step, (uint32_t)(step >> 32), 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
 }
+// Another stream of the same counter space (stream layout: include/narde_b200.h, narde_segment_sample)
+NHD U4 stream_random(uint64_t seed, uint32_t env, uint64_t step, uint32_t stream) {
+  return philox4x32_10(env, (uint32_t)step, (uint32_t)(step >> 32), stream, (uint32_t)seed, (uint32_t)(seed >> 32));
+}
 // narde_env.py:111-117: roll one die each until they differ; the higher roll makes White start
 NHD int opening_player(uint64_t seed, uint32_t env, uint64_t step) {
   for (uint32_t attempt = 0; attempt < 32; attempt++) {

@@ -832,15 +832,19 @@ __global__ void __launch_bounds__(kThreads) k_afterstates_scan(const uint4* lo, 
 // with a large capacity, scored and arg-maxed like the main batch; k_scatter_choice puts the results back.
 // ctrl: [0] overflowing envs seen (all of them, also beyond m), [1] finished CTAs, [2] envs not covered so far (total).
 // Slots beyond the gathered ones are marked finished games (no legal action, no afterstate rows) by the last CTA.
+// act_override (optional): zeroed for every env, so that the turn starts without an override that an earlier choice left
+// unconsumed (k_scatter_choice writes this turn's overrides after this kernel).
 __global__ void __launch_bounds__(kThreads) k_gather_overflow(const uint4* lo, const uint4* hi, const uint8_t* dice,
                                                              const uint8_t* overflow, int64_t n, int m, uint4* sub_lo,
-                                                             uint4* sub_hi, uint8_t* sub_dice, int32_t* sub_idx, int32_t* ctrl) {
+                                                             uint4* sub_hi, uint8_t* sub_dice, int32_t* sub_idx, int32_t* ctrl,
+                                                             uint64_t* act_override) {
   __shared__ int s_last;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   // The k-th gathered env goes to slot (k mod T) * 32 + k / T, T = m / 32: consecutive entries land in different 32-slot
   // tiles, so the few hundred long lists are spread over all CTAs of the side batch's kernels instead of filling the
   // first ones (contiguous slots: 136 + 140 us for the side enumeration and its afterstate rows; spread: see DESIGN 9).
   const int T = m >> 5;
+  if (i < n && act_override) act_override[i] = 0ull;
   if (i < n && overflow[i]) {
     const int seq = atomicAdd(&ctrl[0], 1);
     if (seq < m) {
@@ -897,11 +901,46 @@ __global__ void __launch_bounds__(256) k_scatter_choice(const int32_t* sub_choic
   if (blockIdx.x == 0 && threadIdx.x == 0) ctrl[0] = 0;  // ready for the next turn's gather (nothing here reads it)
 }
 
+// Exploration of narde_segment_sample (the Philox streams and the rule: include/narde_b200.h).  The parameters are read
+// from device memory, so a captured CUDA graph picks up new values without a recapture.
+struct SampleArgs {
+  const float* params;      // {epsilon, inv_temperature}
+  const int32_t* env_idx;   // slot -> env index (NULL: slot i is env i); a slot of -1 is skipped
+  int64_t env_base;
+  uint64_t seed, step;
+  const uint64_t* step_dev;  // the turn number on the device (overrides step), as in StepFullArgs
+};
+
+// Per env: its global id, the turn number and 1 / temperature; returns the explored index (the env's own uniform
+// policy over its c actions, pick_from_word), -1 when the env does not explore, -2 for a skipped slot.
+__device__ __forceinline__ int sample_prologue(const SampleArgs& S, int64_t i, int c, uint32_t* env, uint64_t* step,
+                                               float* inv_tau) {
+  int64_t e = i;
+  if (S.env_idx) {
+    e = S.env_idx[i];
+    if (e < 0) return -2;
+  }
+  *env = (uint32_t)(S.env_base + e);
+  *step = S.step_dev ? *S.step_dev : S.step;
+  *inv_tau = S.params[1];
+  if (c == 0) return -1;
+  const uint32_t below = (uint32_t)(S.params[0] * 16777216.0f);  // floor(eps * 2^24), exact for eps in [0, 1]
+  if ((stream_random(S.seed, *env, *step, 2u).x >> 8) >= below) return -1;
+  return (int)mulhi32(turn_random(S.seed, *env, *step).z, (uint32_t)c);
+}
+// Gumbel noise of action k: u = ((w >> 9) + 1/2) / 2^23 lies strictly inside (0, 1) in float32, so G is finite
+__device__ __forceinline__ float gumbel(uint64_t seed, uint32_t env, uint64_t step, int k) {
+  const float u = ((float)(stream_random(seed, env, step, 3u + ((uint32_t)k << 8)).x >> 9) + 0.5f) * 0x1p-23f;
+  return -logf(-logf(u));
+}
+
 // The same for long segments (the side batch: lists of hundreds to thousands of actions): a warp per env, lanes stride over
 // the segment (coalesced), the (value, index) pairs reduced by shuffles -- a thread per env walks such a segment alone.
+// kSample: narde_segment_sample (each lane draws the noise of its own actions); otherwise greedy.
+template <bool kSample>
 __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* score, const int64_t* offsets, const int32_t* counts,
                                                                  const uint4* hi, int64_t n, int cap, int mode, int32_t* idx_out,
-                                                                 float* best_out) {
+                                                                 float* best_out, SampleArgs S) {
   const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (i >= n) return;  // (whole warps leave together)
@@ -913,10 +952,27 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* s
     const uint32_t meta = hi[i].z;
     if ((int)(int8_t)((meta >> 16) & 0xFF) != 1) sign = -1.0f;
   }
+  uint32_t env = 0;
+  uint64_t step = 0;
+  float inv_tau = 0.0f;
+  if constexpr (kSample) {
+    const int x = sample_prologue(S, i, c, &env, &step, &inv_tau);  // (the same for every lane)
+    if (x == -2) return;
+    if (x >= 0) {
+      if (lane == 0) {
+        idx_out[i] = x;
+        if (best_out) best_out[i] = score[base + x];
+      }
+      return;
+    }
+  }
   float best = 0.0f;
   int best_k = 0x7FFFFFFF;
   for (int k = lane; k < c; k += 32) {
-    const float v = sign * score[base + k];
+    float v = sign * score[base + k];
+    if constexpr (kSample) {
+      if (inv_tau > 0.0f) v = v * inv_tau + gumbel(S.seed, env, step, k);
+    }
     if (best_k == 0x7FFFFFFF || v > best) {  // strictly greater: the lowest index of a lane's maximum stays
       best = v;
       best_k = k;
@@ -933,15 +989,17 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* s
   }
   if (lane == 0) {
     idx_out[i] = c ? best_k : 0;
-    if (best_out) best_out[i] = c ? sign * best : 0.0f;
+    if (best_out) best_out[i] = c ? (kSample ? score[base + best_k] : sign * best) : 0.0f;
   }
 }
 
 // Greedy choice per env over its segment of afterstate scores: mode 0 = maximise; mode 1 = WHITE
 // maximises, BLACK minimises (a value net that scores positions for WHITE).  Ties -> lowest index.
+// kSample: narde_segment_sample's epsilon-greedy / Gumbel-max choice instead.
+template <bool kSample>
 __global__ void __launch_bounds__(kThreads) k_segment_argmax(const float* score, const int64_t* offsets, const int32_t* counts,
                                                             const uint4* hi, int64_t n, int cap, int mode, int32_t* idx_out,
-                                                            float* best_out) {
+                                                            float* best_out, SampleArgs S) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   int c = counts[i];
@@ -952,17 +1010,32 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax(const float* score,
     const uint32_t meta = hi[i].z;
     if ((int)(int8_t)((meta >> 16) & 0xFF) != 1) sign = -1.0f;
   }
+  uint32_t env = 0;
+  uint64_t step = 0;
+  float inv_tau = 0.0f;
+  if constexpr (kSample) {
+    const int x = sample_prologue(S, i, c, &env, &step, &inv_tau);
+    if (x == -2) return;
+    if (x >= 0) {
+      idx_out[i] = x;
+      if (best_out) best_out[i] = score[base + x];
+      return;
+    }
+  }
   int best_k = 0;
   float best = 0.0f;
   for (int k = 0; k < c; k++) {
     float v = sign * score[base + k];
+    if constexpr (kSample) {
+      if (inv_tau > 0.0f) v = v * inv_tau + gumbel(S.seed, env, step, k);
+    }
     if (k == 0 || v > best) {
       best = v;
       best_k = k;
     }
   }
   idx_out[i] = best_k;
-  if (best_out) best_out[i] = c ? sign * best : 0.0f;
+  if (best_out) best_out[i] = c ? (kSample ? score[base + best_k] : sign * best) : 0.0f;
 }
 
 // Trainer-compatible action codes (train_deepq_pytorch.py:432-437,495-507,752-761): for every stored legal
@@ -1036,6 +1109,18 @@ __global__ void k_advance_counter(uint64_t* ctr) { *ctr += 1; }
 
 inline int grid_for(int64_t n) { return (int)((n + kThreads - 1) / kThreads); }
 inline int launch_status() { return (int)cudaGetLastError(); }
+
+template <bool kSample>
+int launch_segment(const float* score, const int64_t* offsets, const int32_t* counts, const void* hi, int64_t n, int cap, int mode,
+                   int32_t* idx_out, float* best_out, const SampleArgs& S, void* stream) {
+  if (cap > 128)  // long segments: a warp per env
+    k_segment_argmax_warp<kSample><<<grid_for(n * 32), kThreads, 0, (cudaStream_t)stream>>>(score, offsets, counts, (const uint4*)hi,
+                                                                                             n, cap, mode, idx_out, best_out, S);
+  else
+    k_segment_argmax<kSample><<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>(score, offsets, counts, (const uint4*)hi, n, cap,
+                                                                                  mode, idx_out, best_out, S);
+  return launch_status();
+}
 inline bool aligned16(const void* p) { return (((uintptr_t)p) & 15u) == 0; }
 
 }  // namespace
@@ -1298,15 +1383,22 @@ int narde_afterstates_scan(const void* lo, const void* hi, const uint64_t* actio
   return launch_status();
 }
 
-int narde_gather_overflow(const void* lo, const void* hi, const uint8_t* dice, const uint8_t* overflow, int64_t n, int32_t m,
-                          void* sub_lo, void* sub_hi, uint8_t* sub_dice, int32_t* sub_idx, int32_t* ctrl, void* stream) {
+int narde_gather_overflow_clear(const void* lo, const void* hi, const uint8_t* dice, const uint8_t* overflow, int64_t n,
+                                int32_t m, void* sub_lo, void* sub_hi, uint8_t* sub_dice, int32_t* sub_idx, int32_t* ctrl,
+                                uint64_t* act_override, void* stream) {
   if (n == 0) return 0;
   if (n < 0 || m <= 0 || (m & 31) != 0 || !lo || !hi || !dice || !overflow || !sub_lo || !sub_hi || !sub_dice || !sub_idx || !ctrl) return -1;
   if (!aligned16(lo) || !aligned16(hi) || !aligned16(sub_lo) || !aligned16(sub_hi)) return -1;
   if ((((uintptr_t)dice) & 1u) != 0 || (((uintptr_t)sub_dice) & 1u) != 0) return -1;
   k_gather_overflow<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>((const uint4*)lo, (const uint4*)hi, dice, overflow, n, m,
-                                                                        (uint4*)sub_lo, (uint4*)sub_hi, sub_dice, sub_idx, ctrl);
+                                                                        (uint4*)sub_lo, (uint4*)sub_hi, sub_dice, sub_idx, ctrl,
+                                                                        act_override);
   return launch_status();
+}
+
+int narde_gather_overflow(const void* lo, const void* hi, const uint8_t* dice, const uint8_t* overflow, int64_t n, int32_t m,
+                          void* sub_lo, void* sub_hi, uint8_t* sub_dice, int32_t* sub_idx, int32_t* ctrl, void* stream) {
+  return narde_gather_overflow_clear(lo, hi, dice, overflow, n, m, sub_lo, sub_hi, sub_dice, sub_idx, ctrl, nullptr, stream);
 }
 
 int narde_scatter_choice(const int32_t* sub_choice, const float* sub_value, const int32_t* sub_idx, const int32_t* sub_counts_eff,
@@ -1349,13 +1441,16 @@ int narde_segment_argmax(const float* score, const int64_t* offsets, const int32
                          int32_t cap, int32_t mode, int32_t* idx_out, float* best_out, void* stream) {
   if (n == 0) return 0;
   if (n < 0 || cap <= 0 || !score || !offsets || !counts || !hi || !idx_out || !aligned16(hi)) return -1;
-  if (cap > 128)  // long segments: a warp per env
-    k_segment_argmax_warp<<<grid_for(n * 32), kThreads, 0, (cudaStream_t)stream>>>(score, offsets, counts, (const uint4*)hi, n, cap,
-                                                                                   mode, idx_out, best_out);
-  else
-    k_segment_argmax<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>(score, offsets, counts, (const uint4*)hi, n, cap, mode,
-                                                                         idx_out, best_out);
-  return launch_status();
+  return launch_segment<false>(score, offsets, counts, hi, n, cap, mode, idx_out, best_out, SampleArgs{}, stream);
+}
+
+int narde_segment_sample(const float* score, const int64_t* offsets, const int32_t* counts, const void* hi, int64_t n,
+                         int32_t cap, int32_t mode, const int32_t* env_idx, int64_t env_base, uint64_t seed, uint64_t step,
+                         const uint64_t* step_dev, const float* params, int32_t* idx_out, float* value_out, void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || cap <= 0 || !score || !offsets || !counts || !hi || !params || !idx_out || !aligned16(hi)) return -1;
+  const SampleArgs S = {params, env_idx, env_base, seed, step, step_dev};
+  return launch_segment<true>(score, offsets, counts, hi, n, cap, mode, idx_out, value_out, S, stream);
 }
 
 int narde_action_codes(const uint64_t* actions, const int32_t* counts, int64_t n, int32_t cap, int32_t* codes, void* stream) {

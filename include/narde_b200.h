@@ -243,6 +243,12 @@ int narde_afterstates_scan(const void *lo, const void *hi, const uint64_t *actio
 int narde_gather_overflow(const void *lo, const void *hi, const uint8_t *dice, const uint8_t *overflow, int64_t n,
                           int32_t m, void *sub_lo, void *sub_hi, uint8_t *sub_dice, int32_t *sub_idx, int32_t *ctrl,
                           void *stream);
+/* narde_gather_overflow that also zeroes act_override[i] ([n] u64, may be NULL) for every environment, so that a turn
+ * starts with no override that an earlier choice left unconsumed (a narde_scatter_choice whose choice was then played by
+ * narde_step_full instead of narde_step_chosen); this turn's narde_scatter_choice writes its overrides after it. */
+int narde_gather_overflow_clear(const void *lo, const void *hi, const uint8_t *dice, const uint8_t *overflow, int64_t n,
+                                int32_t m, void *sub_lo, void *sub_hi, uint8_t *sub_dice, int32_t *sub_idx, int32_t *ctrl,
+                                uint64_t *act_override, void *stream);
 int narde_scatter_choice(const int32_t *sub_choice, const float *sub_value, const int32_t *sub_idx,
                          const int32_t *sub_counts_eff, const int32_t *sub_counts, int32_t m, int32_t cap,
                          int32_t *choice, float *value, int32_t *ctrl, const uint64_t *sub_actions,
@@ -267,6 +273,33 @@ int narde_step_chosen(void *lo, void *hi, int64_t n, int64_t env_base, uint64_t 
 int narde_segment_argmax(const float *score, const int64_t *offsets, const int32_t *counts, const void *hi,
                          int64_t n, int32_t cap, int32_t mode, int32_t *idx_out, float *best_out,
                          void *stream);
+
+/* Exploring policy over the same segments (epsilon-greedy and softmax, exact and reproducible on the host).
+ * Every random word is a Philox4x32-10 word with key = seed and counter = (g, step_lo, step_hi, stream), where g is the
+ * environment's global id and step the turn number its dice were rolled with (narde_roll_dice).  The low byte of
+ * `stream` tells the uses apart:
+ *   0             the dice (words x, y) and the environment's own uniform action (word z, narde_step_full)
+ *   1 + (a << 8)  the opening roll-off, attempt a (narde_reset)
+ *   2             the exploration coin (word x)
+ *   3 + (k << 8)  the Gumbel noise of action k of the canonical list (word x)
+ * With params = {epsilon, inv_temperature} (device float32[2], read by the kernel: a captured graph picks up new values):
+ *   - environment g explores iff (coin >> 8) < floor(epsilon * 2^24) (epsilon 1: always, 0: never); it then plays
+ *     k = (z * c) >> 32 over its c = min(counts[i], cap) actions, where z is word z of stream 0: exactly the uniform
+ *     choice of narde_step_full when c is the whole list;
+ *   - otherwise, with inv_temperature > 0, k = argmax_k (sign * score_k * inv_temperature + G_k), G_k = -log(-log(u_k)),
+ *     u_k = ((w_k >> 9) + 0.5) * 2^-23 (strictly inside (0, 1) in float32): Gumbel-max, an exact sample of
+ *     softmax(sign * score / temperature); sign = -1 for BLACK to move in mode 1, else +1; ties: lowest index;
+ *   - otherwise the arg-max of narde_segment_argmax, bit for bit (zero parameters: the greedy choice).
+ * value_out (may be NULL) receives score[offsets[i] + k] of the chosen k (0 for an empty segment).
+ * env_idx (may be NULL): [n] i32, the environment of slot i (g = env_base + env_idx[i]; a side batch of
+ * narde_gather_overflow); slots of -1 are skipped.  NULL: g = env_base + i.  step_dev (may be NULL) overrides `step`
+ * with the device-resident turn number, as in narde_step_full.  A side batch sampled with the same rule over the whole
+ * list uses the same coin and, per index k, the same noise as the main pass: narde_scatter_choice's override of the
+ * main pass's choice is an exact sample over every legal action. */
+int narde_segment_sample(const float *score, const int64_t *offsets, const int32_t *counts, const void *hi,
+                         int64_t n, int32_t cap, int32_t mode, const int32_t *env_idx, int64_t env_base,
+                         uint64_t seed, uint64_t step, const uint64_t *step_dev, const float *params,
+                         int32_t *idx_out, float *value_out, void *stream);
 
 /* Trainer-compatible action codes for every stored legal turn action: the reference's (move1_code,
  * move2_code) pairs (train_deepq_pytorch.py:432-437,495-507; action_to_idx :752-761): code = from*24 + to,
