@@ -866,12 +866,7 @@ struct BlockStep {
     if (!valid) return;
     uint8_t kind = sh.kind[tid];
     if (kind == K_DONE) {
-      if (A.counts) A.counts[i] = 0;
-      if (A.dice_out) A.dice_out[2 * i] = A.dice_out[2 * i + 1] = 0;
-      if (A.chosen) A.chosen[i] = ACT_EMPTY;
-      if (A.reward) A.reward[i] = 0.0f;
-      if (A.done) A.done[i] = (A.flags & F_ENUMERATE_ONLY) ? 0 : 1;
-      if (A.truncated) A.truncated[i] = 0;
+      idle_outputs(i, A);
       L.result = DONE_TERMINATED;  // a finished game without auto-reset stays terminated
       return;
     }

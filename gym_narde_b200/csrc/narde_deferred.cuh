@@ -600,6 +600,19 @@ struct ExactStep {
       if (survivors) break;
     }
   }
+  // ---- after solve, one thread: the chosen action played on st (a copy of sh.st), then the turn's completion ---------
+  static NHD void complete(const Sh& sh, State& st, int64_t i, const StepFullArgs& A, StepFullLocal& L) {
+    if (sh.count && !(A.flags & F_ENUMERATE_ONLY)) {  // apply_action, rolled up (code size)
+#pragma unroll 1
+      for (int k = 0; k < 4; k++) {
+        const uint32_t h = (uint32_t)(sh.chosen >> (16 * k)) & 0xFFFFu;
+        if (h == 0xFFFFu) break;
+        apply_half_move(st, sh.player, (int)(h & 0xFF), (h >> 8) == 255u ? -1 : (int)(h >> 8));
+      }
+    }
+    complete_env(st, i, A, sh.player, sh.count, sh.chosen, sh.d1, sh.d2, L, false);
+    L.clamped = A.action_idx ? index_was_clamped(A, (uint32_t)A.action_idx[i], sh.count) : 0;
+  }
 };
 
 }  // namespace narde

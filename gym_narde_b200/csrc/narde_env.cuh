@@ -2,6 +2,7 @@
 // The CUDA kernels (narde_kernels.cu) wrap these with coalesced state loads/stores; the
 // test-only host harness (tests/hostsim/) wraps the same bodies in plain loops.
 #pragma once
+#include "../../include/narde_b200.h"
 #include "narde_core.cuh"
 
 namespace narde {
@@ -107,6 +108,32 @@ struct StepFullArgs {
   uint32_t* mirror_compact;
 };
 
+// The arguments of a step call over n envs, set by name; the optional parts (deferral, mirrors) stay zero
+inline StepFullArgs step_args(int64_t n, int64_t env_base, uint64_t seed, uint64_t step, const uint8_t* dice_in,
+                              const int32_t* action_idx, int cap, uint64_t* actions, int32_t* counts, uint8_t* dice_out,
+                              uint64_t* chosen, float* reward, uint8_t* done, uint8_t* truncated, int flags,
+                              int max_episode_steps, const uint64_t* step_dev) {
+  StepFullArgs A = {};
+  A.env_base = env_base;
+  A.seed = seed;
+  A.step = step;
+  A.dice_in = dice_in;
+  A.action_idx = action_idx;
+  A.cap = cap;
+  A.actions = cap > 0 ? actions : nullptr;
+  A.counts = counts;
+  A.dice_out = dice_out;
+  A.chosen = chosen;
+  A.reward = reward;
+  A.done = done;
+  A.truncated = truncated;
+  A.flags = flags;
+  A.max_episode_steps = max_episode_steps;
+  A.step_dev = step_dev;
+  A.list_cap = n;
+  return A;
+}
+
 // state (+ result bits) -> the 5 words of the compact host record
 NHD void pack_compact(const State& s, int result, uint32_t out[5]) {
   uint64_t a = 0, b = 0;  // points 0..11 / 12..23, 5-bit two's complement each
@@ -147,6 +174,22 @@ struct StepFullLocal {  // per-env contributions to the stats vector
   int clamped;  // the caller's action index was out of range (set by the kernels after complete_env)
   int result;   // bit 0 terminated, bit 1 truncated, bits 2-3 the reward (0, 1, 2): the NARDE_PACK_RESULT byte
 };
+// One env's contributions added to the stats vector: atomics on the device, plain adds on the host
+NHD void stats_add_env(int64_t* stats, const StepFullLocal& L) {
+  int v[6] = {L.finished, L.white_win, L.black_win, L.mars, L.ep_len, L.count};
+#if defined(__CUDA_ARCH__)
+  for (int k = 0; k < 6; k++)
+    if (v[k]) atomicAdd(reinterpret_cast<unsigned long long*>(stats + k), (unsigned long long)v[k]);
+  if (L.count) atomicMax(reinterpret_cast<long long*>(stats + NARDE_STAT_MAX_ACTIONS), (long long)L.count);
+  if (L.overflow) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_OVERFLOWS), 1ull);
+  if (L.clamped) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_CLAMPED_ACTIONS), 1ull);
+#else
+  for (int k = 0; k < 6; k++) stats[k] += v[k];
+  if (L.count > stats[NARDE_STAT_MAX_ACTIONS]) stats[NARDE_STAT_MAX_ACTIONS] = L.count;
+  stats[NARDE_STAT_OVERFLOWS] += L.overflow;
+  stats[NARDE_STAT_CLAMPED_ACTIONS] += L.clamped;
+#endif
+}
 // SURVEY 8b "Errors": an out-of-range index never raises (the reference's step forfeits silently, narde_env.py:63);
 // it is clamped and counted
 NHD int index_was_clamped(const StepFullArgs& A, uint32_t word, uint32_t count) {
@@ -233,6 +276,17 @@ NHD void step_full_env(State& s, int64_t i, const StepFullArgs& A, StepFullLocal
   if (A.reward) A.reward[i] = rew;
   if (A.done) A.done[i] = (bits & DONE_TERMINATED) ? 1 : 0;
   if (A.truncated) A.truncated[i] = (bits & DONE_TRUNCATED) ? 1 : 0;
+}
+
+// Outputs of a finished game without auto-reset, which stays as it is: no action, no reward, still terminated
+// (under F_ENUMERATE_ONLY the "done" output carries the overflow flag: 0)
+NHD void idle_outputs(int64_t i, const StepFullArgs& A) {
+  if (A.counts) A.counts[i] = 0;
+  if (A.dice_out) A.dice_out[2 * i] = A.dice_out[2 * i + 1] = 0;
+  if (A.chosen) A.chosen[i] = ACT_EMPTY;
+  if (A.reward) A.reward[i] = 0.0f;
+  if (A.done) A.done[i] = (A.flags & F_ENUMERATE_ONLY) ? 0 : 1;
+  if (A.truncated) A.truncated[i] = 0;
 }
 
 // End-of-turn completion shared by the kernels: apply, termination / reward / switch, auto-reset,

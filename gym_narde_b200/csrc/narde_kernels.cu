@@ -103,6 +103,40 @@ __device__ __forceinline__ void write_obs198_cta(const State* sm, const float4* 
   }
 }
 
+// The stats contributions of a warp's envs: a warp-level reduction, one atomic per warp per slot that is non-zero
+__device__ __forceinline__ void stats_flush_warp(int64_t* stats, const StepFullLocal& L, int tid) {
+  unsigned full = 0xFFFFFFFFu;
+  int v[6] = {L.finished, L.white_win, L.black_win, L.mars, L.ep_len, L.count};
+  int mx = L.count, ov = L.overflow, cl = L.clamped;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+    for (int k = 0; k < 6; k++) v[k] += __shfl_xor_sync(full, v[k], o);
+    mx = max(mx, __shfl_xor_sync(full, mx, o));
+    ov += __shfl_xor_sync(full, ov, o);
+    cl += __shfl_xor_sync(full, cl, o);
+  }
+  if ((tid & 31) == 0) {
+#pragma unroll
+    for (int k = 0; k < 6; k++)
+      if (v[k]) atomicAdd(reinterpret_cast<unsigned long long*>(stats + k), (unsigned long long)v[k]);
+    if (mx) atomicMax(reinterpret_cast<long long*>(stats + NARDE_STAT_MAX_ACTIONS), (long long)mx);
+    if (ov) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_OVERFLOWS), (unsigned long long)ov);
+    if (cl) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_CLAMPED_ACTIONS), (unsigned long long)cl);
+  }
+}
+
+// CTA writer of obs24 rows (narde_env.py:24-25): 24 int32 per env as contiguous words.  sm[] holds the CTA's states,
+// rows [row0, row0+rows); the CTA must be synchronised before the call.
+__device__ __forceinline__ void write_obs24_cta(const State* sm, int rows, int64_t row0, int32_t* o24) {
+  int32_t* base = o24 + row0 * 24;
+  for (int j = threadIdx.x; j < rows * 24; j += blockDim.x) {
+    int e = j / 24, k = j - e * 24;
+    const State& s = sm[e];
+    base[j] = s.turn() == 1 ? s.point(k) : -s.point(k < 12 ? k + 12 : k - 12);
+  }
+}
+
 __global__ void __launch_bounds__(kThreads) k_reset(uint4* lo, uint4* hi, const uint8_t* mask, int64_t n, int64_t env_base,
                                                    uint64_t seed, uint64_t step) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -141,15 +175,7 @@ __global__ void __launch_bounds__(kThreads) k_step_ref(uint4* lo, uint4* hi, con
   }
   if (!o24) return;
   __syncthreads();
-  int rows = (int)min((int64_t)blockDim.x, n - row0);
-  // narde_env.py:24-25: 24 int32 per env, written as contiguous words by the CTA
-  int32_t* base = o24 + row0 * 24;
-  for (int j = threadIdx.x; j < rows * 24; j += blockDim.x) {
-    int e = j / 24, k = j - e * 24;
-    const State& s = sm[e];
-    int v = s.turn() == 1 ? s.point(k) : -s.point(k < 12 ? k + 12 : k - 12);
-    base[j] = v;
-  }
+  write_obs24_cta(sm, (int)min((int64_t)blockDim.x, n - row0), row0, o24);
 }
 
 __global__ void __launch_bounds__(kThreads) k_enumerate(const uint4* lo, const uint4* hi, const uint8_t* dice, int64_t n, int cap,
@@ -179,28 +205,7 @@ __global__ void __launch_bounds__(kThreads) k_step_full(uint4* lo, uint4* hi, in
     if (A.mirror_lo) st_state((uint4*)A.mirror_lo, (uint4*)A.mirror_hi, i, s);
     sm[threadIdx.x] = s;
   }
-  if (stats) {
-    // warp-level reduction, one atomic per warp per slot that is non-zero
-    unsigned full = 0xFFFFFFFFu;
-    int v[6] = {L.finished, L.white_win, L.black_win, L.mars, L.ep_len, L.count};
-    int mx = L.count, ov = L.overflow, cl = L.clamped;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int k = 0; k < 6; k++) v[k] += __shfl_xor_sync(full, v[k], o);
-      mx = max(mx, __shfl_xor_sync(full, mx, o));
-      ov += __shfl_xor_sync(full, ov, o);
-      cl += __shfl_xor_sync(full, cl, o);
-    }
-    if ((threadIdx.x & 31) == 0) {
-#pragma unroll
-      for (int k = 0; k < 6; k++)
-        if (v[k]) atomicAdd(reinterpret_cast<unsigned long long*>(stats + k), (unsigned long long)v[k]);
-      if (mx) atomicMax(reinterpret_cast<long long*>(stats + NARDE_STAT_MAX_ACTIONS), (long long)mx);
-      if (ov) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_OVERFLOWS), (unsigned long long)ov);
-      if (cl) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_CLAMPED_ACTIONS), (unsigned long long)cl);
-    }
-  }
+  if (stats) stats_flush_warp(stats, L, threadIdx.x);
   if (!obs198) return;
   __shared__ float4 lut[16];
   obs_lut_init(lut);
@@ -228,10 +233,7 @@ __global__ void __launch_bounds__(kThreads) k_step_chosen(uint4* lo, uint4* hi, 
   if (i < n) {
     State s = ld_state(lo, hi, i);
     if (s.flags() & FLAG_DONE) {  // a finished game without auto-reset stays as it is (BlockStep::ph_finish, K_DONE)
-      if (A.chosen) A.chosen[i] = ACT_EMPTY;
-      if (A.reward) A.reward[i] = 0.0f;
-      if (A.done) A.done[i] = 1;
-      if (A.truncated) A.truncated[i] = 0;
+      idle_outputs(i, A);
     } else {
       const int count = counts[i];
       uint64_t act = ACT_EMPTY;
@@ -251,27 +253,7 @@ __global__ void __launch_bounds__(kThreads) k_step_chosen(uint4* lo, uint4* hi, 
     }
     sm[threadIdx.x] = s;
   }
-  if (stats) {
-    unsigned full = 0xFFFFFFFFu;
-    int v[6] = {L.finished, L.white_win, L.black_win, L.mars, L.ep_len, L.count};
-    int mx = L.count, ov = L.overflow, cl = L.clamped;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int k = 0; k < 6; k++) v[k] += __shfl_xor_sync(full, v[k], o);
-      mx = max(mx, __shfl_xor_sync(full, mx, o));
-      ov += __shfl_xor_sync(full, ov, o);
-      cl += __shfl_xor_sync(full, cl, o);
-    }
-    if ((threadIdx.x & 31) == 0) {
-#pragma unroll
-      for (int k = 0; k < 6; k++)
-        if (v[k]) atomicAdd(reinterpret_cast<unsigned long long*>(stats + k), (unsigned long long)v[k]);
-      if (mx) atomicMax(reinterpret_cast<long long*>(stats + NARDE_STAT_MAX_ACTIONS), (long long)mx);
-      if (ov) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_OVERFLOWS), (unsigned long long)ov);
-      if (cl) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_CLAMPED_ACTIONS), (unsigned long long)cl);
-    }
-  }
+  if (stats) stats_flush_warp(stats, L, threadIdx.x);
   if (!obs198) return;
   __syncthreads();
   const int rows = (int)min((int64_t)blockDim.x, n - row0);
@@ -426,27 +408,7 @@ __global__ void __launch_bounds__(NT, MINB) k_step_full_v2(uint4* lo, uint4* hi,
     for (int w = tid; w < nrec * 5; w += NT)
       if (!sh.defer[w / 5]) A.mirror_compact[row0 * 5 + w] = stg[w];
   }
-  if (stats) {
-    unsigned full = 0xFFFFFFFFu;
-    int v[6] = {L.finished, L.white_win, L.black_win, L.mars, L.ep_len, L.count};
-    int mx = L.count, ov = L.overflow, cl = L.clamped;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int k = 0; k < 6; k++) v[k] += __shfl_xor_sync(full, v[k], o);
-      mx = max(mx, __shfl_xor_sync(full, mx, o));
-      ov += __shfl_xor_sync(full, ov, o);
-      cl += __shfl_xor_sync(full, cl, o);
-    }
-    if ((tid & 31) == 0) {
-#pragma unroll
-      for (int k = 0; k < 6; k++)
-        if (v[k]) atomicAdd(reinterpret_cast<unsigned long long*>(stats + k), (unsigned long long)v[k]);
-      if (mx) atomicMax(reinterpret_cast<long long*>(stats + NARDE_STAT_MAX_ACTIONS), (long long)mx);
-      if (ov) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_OVERFLOWS), (unsigned long long)ov);
-      if (cl) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_CLAMPED_ACTIONS), (unsigned long long)cl);
-    }
-  }
+  if (stats) stats_flush_warp(stats, L, tid);
   if (!obs198) return;
   __shared__ float4 lut[16];
   obs_lut_init(lut);
@@ -495,16 +457,7 @@ __device__ __forceinline__ void exact_env(TeamExec& ex, ShT& sh, const float4* l
   if (ex.tid == 0) {
     StepFullLocal L;
     State st = sh.st;
-    if (sh.count && !(A.flags & F_ENUMERATE_ONLY)) {  // apply_action, rolled up (code size: see narde_deferred.cuh)
-#pragma unroll 1
-      for (int k = 0; k < 4; k++) {
-        const uint32_t h = (uint32_t)(sh.chosen >> (16 * k)) & 0xFFFFu;
-        if (h == 0xFFFFu) break;
-        apply_half_move(st, sh.player, (int)(h & 0xFF), (h >> 8) == 255u ? -1 : (int)(h >> 8));
-      }
-    }
-    complete_env(st, i, A, sh.player, sh.count, sh.chosen, sh.d1, sh.d2, L, false);
-    L.clamped = A.action_idx ? index_was_clamped(A, (uint32_t)A.action_idx[i], sh.count) : 0;
+    ExactStep<NT>::complete(sh, st, i, A, L);
     sh.st = st;
     if (!(A.flags & F_ENUMERATE_ONLY)) {
       st_state(lo, hi, i, st);
@@ -515,14 +468,7 @@ __device__ __forceinline__ void exact_env(TeamExec& ex, ShT& sh, const float4* l
         for (int k = 0; k < 5; k++) A.mirror_compact[i * 5 + k] = r[k];
       }
     }
-    if (stats) {
-      int v[6] = {L.finished, L.white_win, L.black_win, L.mars, L.ep_len, L.count};
-      for (int k = 0; k < 6; k++)
-        if (v[k]) atomicAdd(reinterpret_cast<unsigned long long*>(stats + k), (unsigned long long)v[k]);
-      if (L.count) atomicMax(reinterpret_cast<long long*>(stats + NARDE_STAT_MAX_ACTIONS), (long long)L.count);
-      if (L.overflow) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_OVERFLOWS), 1ull);
-      if (L.clamped) atomicAdd(reinterpret_cast<unsigned long long*>(stats + NARDE_STAT_CLAMPED_ACTIONS), 1ull);
-    }
+    if (stats) stats_add_env(stats, L);
   }
   ex.run([](int) {});
   ex.mark(9);
@@ -677,13 +623,7 @@ __global__ void __launch_bounds__(kThreads) k_obs24(const uint4* lo, const uint4
   int64_t i = row0 + threadIdx.x;
   if (i < n) sm[threadIdx.x] = ld_state(lo, hi, i);
   __syncthreads();
-  int rows = (int)min((int64_t)blockDim.x, n - row0);
-  int32_t* base = o24 + row0 * 24;
-  for (int j = threadIdx.x; j < rows * 24; j += blockDim.x) {
-    int e = j / 24, k = j - e * 24;
-    const State& s = sm[e];
-    base[j] = s.turn() == 1 ? s.point(k) : -s.point(k < 12 ? k + 12 : k - 12);
-  }
+  write_obs24_cta(sm, (int)min((int64_t)blockDim.x, n - row0), row0, o24);
 }
 
 __global__ void __launch_bounds__(kThreads) k_apply_actions(uint4* lo, uint4* hi, const uint64_t* acts, int64_t n, int flags,
@@ -928,6 +868,46 @@ __device__ __forceinline__ int sample_prologue(const SampleArgs& S, int64_t i, i
   if ((stream_random(S.seed, *env, *step, 2u).x >> 8) >= below) return -1;
   return (int)mulhi32(turn_random(S.seed, *env, *step).z, (uint32_t)c);
 }
+// One env's segment as both segment kernels begin it: the count (clamped to cap), the first row, the sign (mode 1: BLACK
+// minimises) and, when sampling, the env's global id, the turn number and 1 / temperature.
+struct Segment {
+  int c;
+  int64_t base;
+  float sign;
+  uint32_t env;
+  uint64_t step;
+  float inv_tau;
+};
+// Returns false when the env is settled before its scores are read: a skipped slot, or an env that explores (its
+// index and score are stored by the `writer` thread).
+template <bool kSample>
+__device__ __forceinline__ bool segment_begin(Segment& g, const float* score, const int64_t* offsets, const int32_t* counts,
+                                              const uint4* hi, int64_t i, int cap, int mode, const SampleArgs& S, bool writer,
+                                              int32_t* idx_out, float* best_out) {
+  const int c = counts[i];
+  g.c = c < cap ? c : cap;
+  g.base = offsets[i];
+  g.sign = 1.0f;
+  if (mode == 1) {
+    const uint32_t meta = hi[i].z;
+    if ((int)(int8_t)((meta >> 16) & 0xFF) != 1) g.sign = -1.0f;
+  }
+  g.env = 0;
+  g.step = 0;
+  g.inv_tau = 0.0f;
+  if constexpr (kSample) {
+    const int x = sample_prologue(S, i, g.c, &g.env, &g.step, &g.inv_tau);
+    if (x == -2) return false;
+    if (x >= 0) {
+      if (writer) {
+        idx_out[i] = x;
+        if (best_out) best_out[i] = score[g.base + x];
+      }
+      return false;
+    }
+  }
+  return true;
+}
 // Gumbel noise of action k: u = ((w >> 9) + 1/2) / 2^23 lies strictly inside (0, 1) in float32, so G is finite
 __device__ __forceinline__ float gumbel(uint64_t seed, uint32_t env, uint64_t step, int k) {
   const float u = ((float)(stream_random(seed, env, step, 3u + ((uint32_t)k << 8)).x >> 9) + 0.5f) * 0x1p-23f;
@@ -944,34 +924,14 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* s
   const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (i >= n) return;  // (whole warps leave together)
-  int c = counts[i];
-  c = c < cap ? c : cap;
-  const int64_t base = offsets[i];
-  float sign = 1.0f;
-  if (mode == 1) {
-    const uint32_t meta = hi[i].z;
-    if ((int)(int8_t)((meta >> 16) & 0xFF) != 1) sign = -1.0f;
-  }
-  uint32_t env = 0;
-  uint64_t step = 0;
-  float inv_tau = 0.0f;
-  if constexpr (kSample) {
-    const int x = sample_prologue(S, i, c, &env, &step, &inv_tau);  // (the same for every lane)
-    if (x == -2) return;
-    if (x >= 0) {
-      if (lane == 0) {
-        idx_out[i] = x;
-        if (best_out) best_out[i] = score[base + x];
-      }
-      return;
-    }
-  }
+  Segment g;
+  if (!segment_begin<kSample>(g, score, offsets, counts, hi, i, cap, mode, S, lane == 0, idx_out, best_out)) return;
   float best = 0.0f;
   int best_k = 0x7FFFFFFF;
-  for (int k = lane; k < c; k += 32) {
-    float v = sign * score[base + k];
+  for (int k = lane; k < g.c; k += 32) {
+    float v = g.sign * score[g.base + k];
     if constexpr (kSample) {
-      if (inv_tau > 0.0f) v = v * inv_tau + gumbel(S.seed, env, step, k);
+      if (g.inv_tau > 0.0f) v = v * g.inv_tau + gumbel(S.seed, g.env, g.step, k);
     }
     if (best_k == 0x7FFFFFFF || v > best) {  // strictly greater: the lowest index of a lane's maximum stays
       best = v;
@@ -988,8 +948,8 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* s
     }
   }
   if (lane == 0) {
-    idx_out[i] = c ? best_k : 0;
-    if (best_out) best_out[i] = c ? (kSample ? score[base + best_k] : sign * best) : 0.0f;
+    idx_out[i] = g.c ? best_k : 0;
+    if (best_out) best_out[i] = g.c ? (kSample ? score[g.base + best_k] : g.sign * best) : 0.0f;
   }
 }
 
@@ -1002,32 +962,14 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax(const float* score,
                                                             float* best_out, SampleArgs S) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  int c = counts[i];
-  c = c < cap ? c : cap;
-  const int64_t base = offsets[i];
-  float sign = 1.0f;
-  if (mode == 1) {
-    const uint32_t meta = hi[i].z;
-    if ((int)(int8_t)((meta >> 16) & 0xFF) != 1) sign = -1.0f;
-  }
-  uint32_t env = 0;
-  uint64_t step = 0;
-  float inv_tau = 0.0f;
-  if constexpr (kSample) {
-    const int x = sample_prologue(S, i, c, &env, &step, &inv_tau);
-    if (x == -2) return;
-    if (x >= 0) {
-      idx_out[i] = x;
-      if (best_out) best_out[i] = score[base + x];
-      return;
-    }
-  }
+  Segment g;
+  if (!segment_begin<kSample>(g, score, offsets, counts, hi, i, cap, mode, S, true, idx_out, best_out)) return;
   int best_k = 0;
   float best = 0.0f;
-  for (int k = 0; k < c; k++) {
-    float v = sign * score[base + k];
+  for (int k = 0; k < g.c; k++) {
+    float v = g.sign * score[g.base + k];
     if constexpr (kSample) {
-      if (inv_tau > 0.0f) v = v * inv_tau + gumbel(S.seed, env, step, k);
+      if (g.inv_tau > 0.0f) v = v * g.inv_tau + gumbel(S.seed, g.env, g.step, k);
     }
     if (k == 0 || v > best) {
       best = v;
@@ -1035,7 +977,7 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax(const float* score,
     }
   }
   idx_out[i] = best_k;
-  if (best_out) best_out[i] = c ? (kSample ? score[base + best_k] : sign * best) : 0.0f;
+  if (best_out) best_out[i] = g.c ? (kSample ? score[g.base + best_k] : g.sign * best) : 0.0f;
 }
 
 // Trainer-compatible action codes (train_deepq_pytorch.py:432-437,495-507,752-761): for every stored legal
@@ -1226,35 +1168,13 @@ int narde_step_full_mirror(void* lo, void* hi, int64_t n, int64_t env_base, uint
   if (compact && (flags & NARDE_PER_THREAD_KERNEL)) return -1;
   if (n < 0 || cap < 0 || !lo || !hi || !aligned16(lo) || !aligned16(hi)) return -1;
   if (obs198 && (((uintptr_t)obs198) & 7u) != 0) return -1;
-  if (n == 0) return 0;
-  StepFullArgs A;
-  A.env_base = env_base;
-  A.seed = seed;
-  A.step = step;
-  A.dice_in = dice_in;
-  A.action_idx = action_idx;
-  A.cap = cap;
-  A.actions = cap > 0 ? actions : nullptr;
-  A.counts = counts;
-  A.dice_out = dice_out;
-  A.chosen = chosen;
-  A.reward = reward;
-  A.done = done;
-  A.truncated = truncated;
-  A.flags = flags;
-  A.max_episode_steps = max_episode_steps;
-  A.defer_count = nullptr;
-  A.defer_list = nullptr;
-  A.step_dev = step_dev;
-  A.ticket = nullptr;
-  A.arrivals = nullptr;
-  A.n_primary = 0;
-  A.early_trigger = 0;
-  A.list_cap = n;
-  A.last_count = nullptr;
-  A.mirror_lo = compact ? nullptr : mirror_lo;
+  StepFullArgs A = step_args(n, env_base, seed, step, dice_in, action_idx, cap, actions, counts, dice_out, chosen, reward, done,
+                             truncated, flags, max_episode_steps, step_dev);
+  if (compact)
+    A.mirror_compact = reinterpret_cast<uint32_t*>(mirror_lo);
+  else
+    A.mirror_lo = mirror_lo;
   A.mirror_hi = mirror_hi;
-  A.mirror_compact = compact ? reinterpret_cast<uint32_t*>(mirror_lo) : nullptr;
   const bool dev_advance = (flags & NARDE_DEVICE_ADVANCE) != 0;
   if (dev_advance && (!workspace || !step_dev || (flags & (NARDE_PER_THREAD_KERNEL | NARDE_ENUMERATE_ONLY)))) return -1;
   if (flags & NARDE_PER_THREAD_KERNEL) {
@@ -1418,20 +1338,9 @@ int narde_step_chosen(void* lo, void* hi, int64_t n, int64_t env_base, uint64_t 
   if (n < 0 || cap <= 0 || !lo || !hi || !dice || !choice || !actions || !counts || !aligned16(lo) || !aligned16(hi)) return -1;
   if ((((uintptr_t)dice) & 1u) != 0 || (obs198 && (((uintptr_t)obs198) & 7u) != 0)) return -1;
   if (flags & ~(NARDE_REWARD_MOVER12 | NARDE_AUTORESET)) return -1;
-  StepFullArgs A = {};
-  A.env_base = env_base;
-  A.seed = seed;
-  A.step = step;
-  A.dice_in = dice;
-  A.action_idx = choice;
-  A.cap = cap;
-  A.chosen = chosen;
-  A.reward = reward;
-  A.done = done;
-  A.truncated = truncated;
-  A.flags = flags;
-  A.max_episode_steps = max_episode_steps;
-  A.step_dev = step_dev;
+  // (no counts / dice_out: counts, dice and lists are the enumeration's outputs and stay as they are)
+  const StepFullArgs A = step_args(n, env_base, seed, step, dice, choice, cap, nullptr, nullptr, nullptr, chosen, reward, done,
+                                   truncated, flags, max_episode_steps, step_dev);
   k_step_chosen<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>((uint4*)lo, (uint4*)hi, n, A, actions, counts, act_override,
                                                                    obs198, stats);
   return launch_status();

@@ -39,6 +39,10 @@ static void store_state(void* lo, void* hi, int64_t i, const State& s) {
   h[0] = s.w[4]; h[1] = s.w[5]; h[2] = s.meta; h[3] = s.aux;
 }
 
+static void store_obs198(float* obs198, int64_t i, const State& s) {
+  for (int k = 0; k < 99; k++) obs198_pair(s, k, obs198 + 198 * i + 2 * k, obs198 + 198 * i + 2 * k + 1);
+}
+
 extern "C" {
 
 int hs_reset_masked(void* lo, void* hi, const uint8_t* mask, int64_t n, int64_t env_base, uint64_t seed,
@@ -91,7 +95,7 @@ int hs_enumerate(const void* lo, const void* hi, const uint8_t* dice, int64_t n,
 int hs_obs198(const void* lo, const void* hi, int64_t n, float* obs, void*) {
   for (int64_t i = 0; i < n; i++) {
     State s = load_state(lo, hi, i);
-    for (int k = 0; k < 99; k++) obs198_pair(s, k, obs + 198 * i + 2 * k, obs + 198 * i + 2 * k + 1);
+    store_obs198(obs, i, s);
   }
   return 0;
 }
@@ -107,24 +111,15 @@ int hs_step_full(void* lo, void* hi, int64_t n, int64_t env_base, uint64_t seed,
                  const int32_t* action_idx, int32_t cap, uint64_t* actions, int32_t* counts, uint8_t* dice_out,
                  uint64_t* chosen, float* obs198, float* reward, uint8_t* done, uint8_t* truncated, int64_t* stats,
                  int32_t flags, int32_t max_episode_steps, void*) {
-  StepFullArgs A = {env_base, seed, step, dice_in, action_idx, cap, actions, counts, dice_out,
-                    chosen, reward, done, truncated, flags, max_episode_steps, nullptr, nullptr, nullptr};
-  A.ticket = nullptr; A.arrivals = nullptr; A.n_primary = 0; A.early_trigger = 0; A.list_cap = n; A.mirror_lo = A.mirror_hi = nullptr; A.mirror_compact = nullptr;
-  A.last_count = nullptr;
+  const StepFullArgs A = step_args(n, env_base, seed, step, dice_in, action_idx, cap, actions, counts, dice_out, chosen, reward,
+                                   done, truncated, flags, max_episode_steps, nullptr);
   for (int64_t i = 0; i < n; i++) {
     State s = load_state(lo, hi, i);
     StepFullLocal L;
     step_full_env(s, i, A, L);
     store_state(lo, hi, i, s);
-    if (stats) {
-      stats[0] += L.finished; stats[1] += L.white_win; stats[2] += L.black_win; stats[3] += L.mars;
-      stats[4] += L.ep_len; stats[5] += L.count;
-      if (L.count > stats[6]) stats[6] = L.count;
-      stats[7] += L.overflow;
-      stats[8] += L.clamped;   // NARDE_STAT_CLAMPED_ACTIONS
-    }
-    if (obs198)
-      for (int k = 0; k < 99; k++) obs198_pair(s, k, obs198 + 198 * i + 2 * k, obs198 + 198 * i + 2 * k + 1);
+    if (stats) stats_add_env(stats, L);
+    if (obs198) store_obs198(obs198, i, s);
   }
   return 0;
 }
@@ -178,16 +173,8 @@ static void step_full_v2_host(void* lo, void* hi, int64_t n, const StepFullArgs&
       BS::ph_finish(t, sh, valid, row0 + t, A, L);
       if (!valid || sh.defer[t]) continue;
       store_state(lo, hi, row0 + t, sh.st[t]);
-      if (stats) {
-        stats[0] += L.finished; stats[1] += L.white_win; stats[2] += L.black_win; stats[3] += L.mars;
-        stats[4] += L.ep_len; stats[5] += L.count;
-        if (L.count > stats[6]) stats[6] = L.count;
-        stats[7] += L.overflow;
-        stats[8] += L.clamped;   // NARDE_STAT_CLAMPED_ACTIONS
-      }
-      if (obs198)
-        for (int k = 0; k < 99; k++)
-          obs198_pair(sh.st[t], k, obs198 + 198 * (row0 + t) + 2 * k, obs198 + 198 * (row0 + t) + 2 * k + 1);
+      if (stats) stats_add_env(stats, L);
+      if (obs198) store_obs198(obs198, row0 + t, sh.st[t]);
     }
   }
 }
@@ -213,18 +200,10 @@ static void step_deferred_host(void* lo, void* hi, const StepFullArgs& A, float*
     ES::solve(ex, sh, s, i, A);
     StepFullLocal L;
     State st = sh.st;
-    complete_env(st, i, A, sh.player, sh.count, sh.chosen, sh.d1, sh.d2, L);
-    L.clamped = A.action_idx ? index_was_clamped(A, (uint32_t)A.action_idx[i], sh.count) : 0;
+    ES::complete(sh, st, i, A, L);
     store_state(lo, hi, i, st);
-    if (stats) {
-      stats[0] += L.finished; stats[1] += L.white_win; stats[2] += L.black_win; stats[3] += L.mars;
-      stats[4] += L.ep_len; stats[5] += L.count;
-      if (L.count > stats[6]) stats[6] = L.count;
-      stats[7] += L.overflow;
-      stats[8] += L.clamped;   // NARDE_STAT_CLAMPED_ACTIONS
-    }
-    if (obs198)
-      for (int k = 0; k < 99; k++) obs198_pair(st, k, obs198 + 198 * i + 2 * k, obs198 + 198 * i + 2 * k + 1);
+    if (stats) stats_add_env(stats, L);
+    if (obs198) store_obs198(obs198, i, st);
   }
 }
 
@@ -233,10 +212,8 @@ int hs_step_full_v2(void* lo, void* hi, int64_t n, int64_t env_base, uint64_t se
                     const int32_t* action_idx, int32_t cap, uint64_t* actions, int32_t* counts, uint8_t* dice_out,
                     uint64_t* chosen, float* obs198, float* reward, uint8_t* done, uint8_t* truncated, int64_t* stats,
                     int32_t flags, int32_t max_episode_steps, int32_t* workspace, void*) {
-  StepFullArgs A = {env_base, seed, step, dice_in, action_idx, cap, cap > 0 ? actions : nullptr, counts, dice_out,
-                    chosen, reward, done, truncated, flags, max_episode_steps, nullptr, nullptr, nullptr};
-  A.ticket = nullptr; A.arrivals = nullptr; A.n_primary = 0; A.early_trigger = 0; A.list_cap = n; A.mirror_lo = A.mirror_hi = nullptr; A.mirror_compact = nullptr;
-  A.last_count = nullptr;
+  StepFullArgs A = step_args(n, env_base, seed, step, dice_in, action_idx, cap, actions, counts, dice_out, chosen, reward, done,
+                             truncated, flags, max_episode_steps, nullptr);
   if (workspace) {
     for (int k = 0; k < 8; k++) workspace[k] = 0;   // NARDE_WORKSPACE_INTS layout (include/narde_b200.h)
     A.defer_count = workspace;

@@ -19,9 +19,9 @@ _HS_LIB = os.path.join(_HS_DIR, "_build", "libnarde_hostsim.so")
 
 
 def build_hostsim():
-    srcs = [os.path.join(_HS_DIR, "hostsim.cpp"),
-            os.path.join(ROOT, "gym_narde_b200", "csrc", "narde_core.cuh"),
-            os.path.join(ROOT, "gym_narde_b200", "csrc", "narde_env.cuh")]
+    csrc = os.path.join(ROOT, "gym_narde_b200", "csrc")
+    srcs = [os.path.join(_HS_DIR, "hostsim.cpp"), os.path.join(ROOT, "include", "narde_b200.h")] + sorted(
+        os.path.join(csrc, f) for f in os.listdir(csrc) if f.endswith(".cuh"))
     if (not os.path.exists(_HS_LIB)) or any(os.path.getmtime(s) > os.path.getmtime(_HS_LIB) for s in srcs):
         os.makedirs(os.path.dirname(_HS_LIB), exist_ok=True)
         subprocess.check_call(["g++", "-O2", "-fPIC", "-shared", "-std=c++17", "-Wno-unknown-pragmas",

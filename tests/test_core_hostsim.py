@@ -218,3 +218,38 @@ def test_oracle_bulk_trace_equals_stepwise_hostsim(hostsim):
     assert eps >= 150 * 3                                   # every env truncated three times
     turns, _ = P.check_trace_vs_backend(hostsim, 150, 260, 14, flags=1, cap=4)   # mover reward, finished envs idle
     assert turns < 150 * 260
+
+
+def test_hostsim_rebuilds_when_any_included_file_changes(monkeypatch, tmp_path):
+    """The host harness is rebuilt when a file that hostsim.cpp includes, directly or through another header, is newer
+    than the library: a stale library would test old code."""
+    import os
+    import re
+    import subprocess
+
+    import support
+
+    def includes(path, seen):
+        with open(path) as f:
+            names = re.findall(r'^\s*#\s*include\s+"([^"]+)"', f.read(), re.M)
+        for name in names:
+            dep = os.path.realpath(os.path.join(os.path.dirname(path), name))
+            if dep not in seen:
+                seen.add(dep)
+                includes(dep, seen)
+        return seen
+
+    deps = includes(os.path.join(support.ROOT, "tests", "hostsim", "hostsim.cpp"), set())
+    assert any(d.endswith("narde_deferred.cuh") for d in deps)
+    lib = str(tmp_path / "libnarde_hostsim.so")
+    open(lib, "wb").close()
+    monkeypatch.setattr(support, "_HS_LIB", lib)
+    builds = []
+    monkeypatch.setattr(subprocess, "check_call", lambda cmd, **kw: builds.append(cmd))
+    for dep in sorted(deps):
+        # the library is newer than every file but `dep`
+        monkeypatch.setattr(os.path, "getmtime",
+                            lambda p, dep=dep: 1.0 if p == lib else 2.0 if os.path.realpath(p) == dep else 0.0)
+        builds.clear()
+        support.build_hostsim()
+        assert builds, f"a change to {dep} leaves the host harness stale"
