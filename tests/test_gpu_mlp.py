@@ -6,6 +6,8 @@ one floating-point kernel of the path: tolerance (bf16 operands, fp32 accumulate
 import numpy as np
 import pytest
 
+from test_mlp_reference_cpu import bound, ref_q
+
 pytestmark = pytest.mark.gpu
 
 ABS_TOL = 5e-3          # |q_kernel - q_fp32| on Q-values of magnitude ~0.1-0.5 (measured 7e-4; SURVEY 7.10 asks <= 1e-2)
@@ -43,9 +45,16 @@ def test_mlp_matches_fp32_reference_on_real_observations():
             am, rm = q.argmax(1), ref.argmax(1)
             agree = (am == rm).float().mean().item()
             assert agree > ARGMAX_AGREEMENT, agree
-            # where the arg-max differs, the fp32 net itself has the two candidates within the kernel's error
-            gap = ref.gather(1, rm[:, None]) - ref.gather(1, am[:, None])
-            assert gap.max().item() < 2 * ABS_TOL, gap.max().item()
+            # where the arg-max differs, the float64 net itself has the two candidates within the kernel's error
+            # bound of each (a near-tie): gap <= bound[a_kernel] + bound[a_ref]
+            W = tuple(lin.weight.data for lin in (fn[0], fn[2], head))
+            b = tuple(lin.bias.data for lin in (fn[0], fn[2], head))
+            ref64, bnd = ref_q(x, W, b, emulate=False), bound(x, W, b)
+            am, rm = q.argmax(1), ref64.argmax(1)
+            diff = am != rm
+            gap = ref64.gather(1, rm[:, None]) - ref64.gather(1, am[:, None])
+            lim = bnd.gather(1, rm[:, None]) + bnd.gather(1, am[:, None])
+            assert (gap[diff] <= lim[diff]).all(), (gap[diff] - lim[diff]).max().item()
     # exactness of the data path: with bf16-representable weights/inputs the only error is accumulation order
     torch.manual_seed(1)
     xb = torch.randint(0, 2, (512, 198), device="cuda").float()
