@@ -908,6 +908,15 @@ __device__ __forceinline__ bool segment_begin(Segment& g, const float* score, co
   }
   return true;
 }
+// The order of the choice rule (include/narde_b200.h, narde_segment_argmax), shared by both segment kernels, their
+// shuffle reduction and the Gumbel path: (v, k) beats the current (best, best_k) when there is no current choice yet
+// (best_k == kNoChoice), or v is a number and best is NaN, or v > best, or v == best at a lower index.  A NaN never
+// beats a number, so one diverged afterstate does not decide the move, and an all-NaN segment keeps its first index.
+constexpr int kNoChoice = 0x7FFFFFFF;
+__device__ __forceinline__ bool beats(float v, int k, float best, int best_k) {
+  return best_k == kNoChoice || (!isnan(v) && (isnan(best) || v > best || (v == best && k < best_k)));
+}
+
 // Gumbel noise of action k: u = ((w >> 9) + 1/2) / 2^23 lies strictly inside (0, 1) in float32, so G is finite
 __device__ __forceinline__ float gumbel(uint64_t seed, uint32_t env, uint64_t step, int k) {
   const float u = ((float)(stream_random(seed, env, step, 3u + ((uint32_t)k << 8)).x >> 9) + 0.5f) * 0x1p-23f;
@@ -927,13 +936,13 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* s
   Segment g;
   if (!segment_begin<kSample>(g, score, offsets, counts, hi, i, cap, mode, S, lane == 0, idx_out, best_out)) return;
   float best = 0.0f;
-  int best_k = 0x7FFFFFFF;
+  int best_k = kNoChoice;
   for (int k = lane; k < g.c; k += 32) {
     float v = g.sign * score[g.base + k];
     if constexpr (kSample) {
       if (g.inv_tau > 0.0f) v = v * g.inv_tau + gumbel(S.seed, g.env, g.step, k);
     }
-    if (best_k == 0x7FFFFFFF || v > best) {  // strictly greater: the lowest index of a lane's maximum stays
+    if (beats(v, k, best, best_k)) {
       best = v;
       best_k = k;
     }
@@ -942,7 +951,7 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* s
   for (int o = 16; o > 0; o >>= 1) {
     const float ov = __shfl_down_sync(0xFFFFFFFFu, best, o);
     const int ok = __shfl_down_sync(0xFFFFFFFFu, best_k, o);
-    if (ok != 0x7FFFFFFF && (best_k == 0x7FFFFFFF || ov > best || (ov == best && ok < best_k))) {
+    if (ok != kNoChoice && beats(ov, ok, best, best_k)) {
       best = ov;
       best_k = ok;
     }
@@ -954,7 +963,7 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax_warp(const float* s
 }
 
 // Greedy choice per env over its segment of afterstate scores: mode 0 = maximise; mode 1 = WHITE
-// maximises, BLACK minimises (a value net that scores positions for WHITE).  Ties -> lowest index.
+// maximises, BLACK minimises (a value net that scores positions for WHITE).  Ties -> lowest index; NaN: see beats().
 // kSample: narde_segment_sample's epsilon-greedy / Gumbel-max choice instead.
 template <bool kSample>
 __global__ void __launch_bounds__(kThreads) k_segment_argmax(const float* score, const int64_t* offsets, const int32_t* counts,
@@ -964,19 +973,19 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax(const float* score,
   if (i >= n) return;
   Segment g;
   if (!segment_begin<kSample>(g, score, offsets, counts, hi, i, cap, mode, S, true, idx_out, best_out)) return;
-  int best_k = 0;
+  int best_k = kNoChoice;
   float best = 0.0f;
   for (int k = 0; k < g.c; k++) {
     float v = g.sign * score[g.base + k];
     if constexpr (kSample) {
       if (g.inv_tau > 0.0f) v = v * g.inv_tau + gumbel(S.seed, g.env, g.step, k);
     }
-    if (k == 0 || v > best) {
+    if (beats(v, k, best, best_k)) {
       best = v;
       best_k = k;
     }
   }
-  idx_out[i] = best_k;
+  idx_out[i] = g.c ? best_k : 0;
   if (best_out) best_out[i] = g.c ? (kSample ? score[g.base + best_k] : g.sign * best) : 0.0f;
 }
 

@@ -269,7 +269,11 @@ int narde_step_chosen(void *lo, void *hi, int64_t n, int64_t env_base, uint64_t 
 
 /* Greedy policy over each environment's segment of afterstate scores: idx_out[i] = argmax_k
  * score[offsets[i] + k] (mode 0), or argmin when BLACK is to move (mode 1: the net scores positions for
- * WHITE).  best_out (may be NULL): the chosen score.  Ties: lowest index; empty segment: 0. */
+ * WHITE), over k < min(counts[i], cap).  best_out (may be NULL): the chosen score.  Ties: lowest index (-0 and +0 are
+ * equal); empty segment: index 0, score 0.  NaN: a NaN never beats a number, and an all-NaN segment gives index 0 and
+ * its NaN (numpy's nanargmax, unlike torch.argmax, where NaN wins): a net that starts to diverge during training yields
+ * NaN for a few afterstates first, and one such afterstate should neither decide the move nor hide the best defined
+ * score.  The same rule orders the samples of narde_segment_sample. */
 int narde_segment_argmax(const float *score, const int64_t *offsets, const int32_t *counts, const void *hi,
                          int64_t n, int32_t cap, int32_t mode, int32_t *idx_out, float *best_out,
                          void *stream);

@@ -465,31 +465,48 @@ void o_obs198(const int32_t *board_abs, int off_w, int off_b, int player, float 
   out[k++] = player == 1 ? 0.0f : 1.0f;
 }
 
+/* Plays turn action a (NULL: no legal action) for the side to move and finishes the turn: the end-of-game check
+ * (narde_env.py:96) and, unless the game ended, the player switch (:99-100).  Returns the done flag; *rew12 receives
+ * the mover reward of o_check_game_ended. */
+static int o_play_turn(o_env *e, const o_turn_action *a, int32_t *rew12) {
+  const int player = e->current_player;
+  if (a)
+    for (int k = 0; k < a->n_moves; k++)
+      o_execute_rotated_move(&e->game, a->moves[2 * k], a->moves[2 * k + 1], player);
+  *rew12 = 0;
+  const int dn = o_check_game_ended(e, rew12);
+  if (!dn) e->current_player *= -1;
+  return dn;
+}
+
+/* The mover's canonical turn list of e with dice (d1, d2): up to cap entries, returns the full count */
+static int o_enumerate_env(const o_env *e, int d1, int d2, int cap, o_turn_action *out) {
+  int32_t mover[24];
+  const int player = e->current_player;
+  o_get_perspective_board(&e->game, player, mover);
+  return o_turn_enumerate(mover, player == 1 ? e->game.borne_off_white : e->game.borne_off_black, d1, d2,
+                          player == 1 ? e->game.first_turn_white : e->game.first_turn_black, cap, out, 0);
+}
+
 int o_full_step(o_env *e, int d1, int d2, int action_idx, int reward_mode, float *reward,
                 int32_t *done, float *obs198) {
-  int32_t mover[24];
   int player = e->current_player;
-  o_get_perspective_board(&e->game, player, mover);
-  int first_turn = player == 1 ? e->game.first_turn_white : e->game.first_turn_black;
-  int mover_off = player == 1 ? e->game.borne_off_white : e->game.borne_off_black;
   int cap = 4096;
   static __thread o_turn_action *acts = 0; /* per-thread scratch, allocated once */
   if (!acts) acts = (o_turn_action *)malloc((size_t)cap * sizeof(o_turn_action));
-  int n = o_turn_enumerate(mover, mover_off, d1, d2, first_turn, cap, acts, 0);
+  int n = o_enumerate_env(e, d1, d2, cap, acts);
+  const o_turn_action *a = 0;
   if (n > 0) {
     if (action_idx < 0) action_idx = 0;
     if (action_idx >= n) action_idx = n - 1;
-    const o_turn_action *a = &acts[action_idx];
-    for (int k = 0; k < a->n_moves; k++)
-      o_execute_rotated_move(&e->game, a->moves[2 * k], a->moves[2 * k + 1], player);
+    a = &acts[action_idx];
   }
-  int32_t rew12 = 0;
-  int dn = o_check_game_ended(e, &rew12);
+  int32_t rew12;
+  int dn = o_play_turn(e, a, &rew12);
   if (reward_mode == 1)
     *reward = (float)rew12;
   else
     *reward = (dn && player == 1) ? 1.0f : 0.0f; /* README.md:107-108 */
-  if (!dn) e->current_player *= -1;
   *done = dn;
   if (obs198)
     o_obs198(e->game.board, e->game.borne_off_white, e->game.borne_off_black, e->current_player,
@@ -809,6 +826,33 @@ void o_enumerate_batch(const uint8_t *lo, const uint8_t *hi, const uint8_t *dice
     }
     out_count[i] = cnt;
     out_hash[i] = hash;
+  }
+  free(scratch);
+}
+
+/* The afterstate rows of narde_afterstates_scan for n packed positions with given dice: counts_out[i] = the number of
+ * legal turn actions (0 for a finished game), and for each of the first min(count, cap) canonical actions k the packed
+ * action word (actions_out[i*cap + k]) and the state after playing it and finishing the turn as o_full_step does
+ * (as_lo_out / as_hi_out row i*cap + k): terminated bit set when the game ended, episode steps + 1.  Entries at
+ * k >= min(count, cap) are not written. */
+void o_afterstates_batch(const uint8_t *lo, const uint8_t *hi, const uint8_t *dice, int64_t n, int cap,
+                         int32_t *counts_out, uint64_t *actions_out, uint8_t *as_lo_out, uint8_t *as_hi_out) {
+  o_turn_action *scratch = (o_turn_action *)malloc(4096 * sizeof(o_turn_action));
+  for (int64_t i = 0; i < n; i++) {
+    o_env e;
+    int term, esteps;
+    o_unpack_state(lo + 16 * i, hi + 16 * i, &e, &term, &esteps);
+    const int cnt = term ? 0 : o_enumerate_env(&e, dice[2 * i], dice[2 * i + 1], 4096, scratch);
+    counts_out[i] = cnt;
+    const int stored = cnt < cap ? cnt : cap;
+    for (int k = 0; k < stored; k++) {
+      const size_t r = (size_t)i * (size_t)cap + (size_t)k;
+      o_env t = e;
+      int32_t rew12;
+      const int dn = o_play_turn(&t, &scratch[k], &rew12);
+      actions_out[r] = o_pack_action(&scratch[k]);
+      o_pack_state(&t, dn, esteps + 1, as_lo_out + 16 * r, as_hi_out + 16 * r);
+    }
   }
   free(scratch);
 }

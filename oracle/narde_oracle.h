@@ -118,6 +118,11 @@ int64_t o_selfplay_trace(uint64_t seed, uint32_t env_base, int n_envs, int n_ste
 /* get_valid_actions for n packed positions: count + checksum of the first min(count, cap) list entries */
 void o_enumerate_batch(const uint8_t *lo, const uint8_t *hi, const uint8_t *dice, int64_t n, int cap,
                        int32_t *out_count, uint64_t *out_hash);
+/* narde_afterstates_scan's rows for n packed positions: legal-action count, and for each of the first min(count, cap)
+ * canonical actions its u64 word ([n][cap]) and the packed state after it and the end of the turn ([n][cap] x 16 bytes
+ * per plane; the state o_full_step leaves, terminated bit and episode steps as narde_afterstates_scan writes them). */
+void o_afterstates_batch(const uint8_t *lo, const uint8_t *hi, const uint8_t *dice, int64_t n, int cap,
+                         int32_t *counts_out, uint64_t *actions_out, uint8_t *as_lo_out, uint8_t *as_hi_out);
 
 #ifdef __cplusplus
 }

@@ -93,6 +93,8 @@ def lib():
         L.o_selfplay_trace.restype = C.c_int64
         L.o_enumerate_batch.argtypes = [vp, vp, vp, C.c_int64, C.c_int, vp, vp]
         L.o_enumerate_batch.restype = None
+        L.o_afterstates_batch.argtypes = [vp, vp, vp, C.c_int64, C.c_int, vp, vp, vp, vp]
+        L.o_afterstates_batch.restype = None
         L.o_list_weight.argtypes = [C.c_int]
         L.o_list_weight.restype = C.c_uint64
         _lib = L
@@ -327,3 +329,29 @@ def enumerate_batch(lo, hi, dice, cap=64, threads=None):
     with ThreadPoolExecutor(threads) as ex:
         list(ex.map(run, range(0, n, per)))
     return counts, hashes
+
+
+def afterstates_batch(lo, hi, dice, cap=64, threads=None):
+    """o_afterstates_batch on host threads: (counts int32 [n], actions int64 [n, cap], as_lo, as_hi uint8 [n, cap, 16]).
+    Entry (i, k) for k < min(counts[i], cap) is canonical action k of env i and the packed state after it and the end of
+    the turn, as narde_afterstates_scan writes row offsets[i] + k; the other entries are zero."""
+    from concurrent.futures import ThreadPoolExecutor
+    L = lib()
+    lo = np.ascontiguousarray(lo, np.uint8).reshape(-1, 16)
+    hi = np.ascontiguousarray(hi, np.uint8).reshape(-1, 16)
+    dice = np.ascontiguousarray(dice, np.uint8).reshape(-1, 2)
+    n, cap = lo.shape[0], int(cap)
+    counts, actions = np.zeros(n, np.int32), np.zeros((n, cap), np.int64)
+    as_lo, as_hi = np.zeros((n, cap, 16), np.uint8), np.zeros((n, cap, 16), np.uint8)
+    threads = int(threads or os.cpu_count() or 1)
+    per = max(1, -(-n // (threads * 4)))
+
+    def run(b):
+        e = min(b + per, n)
+        L.o_afterstates_batch(lo.ctypes.data + 16 * b, hi.ctypes.data + 16 * b, dice.ctypes.data + 2 * b, e - b, cap,
+                              counts.ctypes.data + 4 * b, actions.ctypes.data + 8 * cap * b,
+                              as_lo.ctypes.data + 16 * cap * b, as_hi.ctypes.data + 16 * cap * b)
+
+    with ThreadPoolExecutor(threads) as ex:
+        list(ex.map(run, range(0, n, per)))
+    return counts, actions, as_lo, as_hi

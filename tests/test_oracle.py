@@ -120,3 +120,74 @@ def test_oracle_vs_live_reference_short():
             assert (obs == oobs).all() and rew == orew and done == odone
             if done:
                 break
+
+
+def _afterstate_positions():
+    """Positions of played games (every phase: selfplay_trace snapshots up to turn 400) and synthetic bear-offs of either
+    colour with one to four checkers left (so that many turns end the game), plus one finished game."""
+    tr = O.selfplay_trace(17, 0, 48, 400, cap=64, max_episode_steps=0, threads=4)
+    lo = tr["lo"][::8].reshape(-1, 16)
+    hi = tr["hi"][::8].reshape(-1, 16)
+    live = (hi[:, 11] & S.FLAG_DONE) == 0
+    lo, hi = lo[live][::3], hi[live][::3]
+    rng = np.random.default_rng(3)
+    boards, off_w, off_b, turn = [], [], [], []
+    for j in range(160):
+        b = np.zeros(24, int)
+        left = int(rng.integers(1, 5))
+        white = j % 2 == 0
+        home = range(0, 6) if white else range(12, 18)       # the mover's home in the absolute frame
+        for _ in range(left):
+            b[rng.choice(list(home))] += 1 if white else -1
+        other = int(rng.integers(0, 15))                     # the other side: 0 off (a mars) or some off
+        b[11 if white else 23] = (-1 if white else 1) * (15 - other)
+        boards.append(b)
+        off_w.append(15 - left if white else other)
+        off_b.append(other if white else 15 - left)
+        turn.append(1 if white else -1)
+    slo, shi = S.pack_states(np.array(boards), off_w=np.array(off_w), off_b=np.array(off_b), turn=np.array(turn),
+                             steps=np.array([(j * 37) % 300 for j in range(160)]))
+    flo, fhi = S.pack_states(np.array(boards[:1]), off_w=off_w[0], off_b=off_b[0], done=True)
+    return np.concatenate([lo, slo, flo]), np.concatenate([hi, shi, fhi])
+
+
+def test_afterstates_batch_equals_full_step():
+    """o_afterstates_batch (the oracle's narde_afterstates_scan rows) against OracleEnv.set_state + full_step(dice, k) for
+    every stored (position, k): doubles and plain dice, bear-offs, game-ending turns, a finished game (no actions), and
+    lists longer than the capacity (only the first `cap` are written, the count is the whole list's)."""
+    lo, hi = _afterstate_positions()
+    n = lo.shape[0]
+    dice = np.array([[1 + (i * 7) % 6, 1 + (i * 11 + i // 6) % 6] for i in range(n)], np.uint8)
+    dice[::5, 1] = dice[::5, 0]                                  # every fifth position rolls doubles
+    cap = 24
+    counts, acts, as_lo, as_hi = O.afterstates_batch(lo, hi, dice, cap=cap, threads=4)
+    want_counts, _ = O.enumerate_batch(lo, hi, dice, cap=cap)
+    assert np.array_equal(counts, want_counts)
+    assert counts[-1] == 0 and not as_lo[-1].any() and not as_hi[-1].any()
+    u = S.unpack_states(lo, hi)
+    pairs = ended = doubles = beyond = 0
+    for i in range(n):
+        stored = min(int(counts[i]), cap)
+        beyond += int(counts[i]) > cap
+        after = S.unpack_states(as_lo[i], as_hi[i])
+        assert not as_lo[i, stored:].any() and not as_hi[i, stored:].any() and not acts[i, stored:].any()
+        player = int(u["turn"][i])
+        mover = u["board"][i] if player == 1 else S.rotate_board(u["board"][i])
+        listed, _ = O.turn_enumerate(mover, u["off_w"][i] if player == 1 else u["off_b"][i], int(dice[i, 0]),
+                                     int(dice[i, 1]), u["first_w"][i] if player == 1 else u["first_b"][i], cap=cap)
+        for k in range(stored):
+            e = O.OracleEnv()
+            e.set_state(u["board"][i], u["off_w"][i], u["off_b"][i], u["first_w"][i], u["first_b"][i], player)
+            _, _, done, cnt = e.full_step(dice[i], k, want_obs=False)
+            assert cnt == counts[i]
+            board, ow, ob, fw, fb, pl = e.state_tuple()
+            got = (tuple(after["board"][k]), after["off_w"][k], after["off_b"][k], int(after["first_w"][k]),
+                   int(after["first_b"][k]), after["turn"][k])
+            assert got == (board, ow, ob, fw, fb, pl), (i, k)
+            assert bool(after["done"][k]) == done and after["steps"][k] == (u["steps"][i] + 1) & 0xFFFF, (i, k)
+            assert S.decode_action(int(acts[i, k]) & 0xFFFFFFFFFFFFFFFF) == [
+                (f, 'off' if t == O.OFF else t) for f, t in listed[k]["moves"]], (i, k)
+            pairs += 1
+            ended += done
+            doubles += int(dice[i, 0] == dice[i, 1])
+    assert pairs > 3000 and ended > 50 and doubles > 500 and beyond > 20, (pairs, ended, doubles, beyond)
