@@ -72,6 +72,11 @@ _SIGNATURES = {
                            _i32, _i32, _vp, _vp], _int),
     "narde_segment_argmax": ([_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp], _int),
     "narde_segment_sample": ([_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _i64, _u64, _u64, _vp, _vp, _vp, _vp, _vp], _int),
+    "narde_segment_topk": ([_vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                            _vp, _vp], _int),
+    "narde_lookahead_expand": ([_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp], _int),
+    "narde_lookahead_reduce": ([_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+                               _int),
     "narde_obs198": ([_vp, _vp, _i64, _vp, _vp], _int),
     "narde_obs24": ([_vp, _vp, _i64, _vp, _vp], _int),
     "narde_apply_actions": ([_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp], _int),
@@ -410,6 +415,78 @@ def segment_sample(score, offsets, counts, hi, cap, mode, env_base, seed, step, 
         _ptr(step_dev, torch.int64, "step_dev", dev, (1,)), _ptr(params, torch.float32, "params", dev, (2,)),
         _ptr(idx_out, torch.int32, "idx_out", dev, (n,)), _ptr(value_out, torch.float32, "value_out", dev, (n,)), _stream())
     _check(rc, "narde_segment_sample")
+
+
+# -- one-ply lookahead (gym_narde_b200/lookahead.py) ----------------------------------------------
+LOOKAHEAD_ROLLS = 21
+LOOKAHEAD_MAX_CANDIDATES = 32
+
+
+def _candidates_k(cand_idx):
+    k = cand_idx.shape[1] if getattr(cand_idx, "dim", lambda: 0)() == 2 else 0
+    if not 1 <= k <= LOOKAHEAD_MAX_CANDIDATES:
+        raise NardeCudaError("cand_idx must be [n, k] with 1 <= k <= %d" % LOOKAHEAD_MAX_CANDIDATES)
+    return k
+
+
+def segment_topk(score, offsets, counts, hi, mode, as_lo, as_hi, actions, cand_idx, cand_score, cand_lo, cand_hi, cand_act,
+                 cand_count, env_idx=None, counts_eff=None, ctrl=None):
+    """narde_segment_topk: the first k = cand_idx.shape[1] actions of each segment score[offsets[i] :][: min(counts[i],
+    cap)] (cap = actions.shape[1]) in the order of segment_argmax's rule, with their scores, afterstate rows (as_lo / as_hi
+    at offsets[i] + index) and action words.  env_idx / counts_eff / ctrl: a side batch's slots overwrite the candidates of
+    the envs they cover (see include/narde_b200.h)."""
+    import torch
+
+    k = _candidates_k(cand_idx)
+    dev, n, m = _device(), hi.shape[0], cand_count.shape[0]
+    acts = _ptr(actions, torch.int64, "actions", dev, (n, _ANY))
+    rc = load().narde_segment_topk(
+        _ptr(score, torch.float32, "score", dev, (_ANY,)), _ptr(offsets, torch.int64, "offsets", dev, (n,)),
+        _ptr(counts, torch.int32, "counts", dev, (n,)), _ptr(hi, torch.uint8, "hi", dev, (n, 16)), n, actions.shape[1], mode, k,
+        _ptr(as_lo, torch.uint8, "as_lo", dev, (_ANY, 16)), _ptr(as_hi, torch.uint8, "as_hi", dev, tuple(as_lo.shape)), acts,
+        _ptr(env_idx, torch.int32, "env_idx", dev, (n,)), _ptr(counts_eff, torch.int32, "counts_eff", dev, (n,)),
+        _ptr(ctrl, torch.int32, "ctrl", dev, (_ANY,), 4), _ptr(cand_idx, torch.int32, "cand_idx", dev, (m, k)),
+        _ptr(cand_score, torch.float32, "cand_score", dev, (m, k)), _ptr(cand_lo, torch.uint8, "cand_lo", dev, (m * k, 16)),
+        _ptr(cand_hi, torch.uint8, "cand_hi", dev, (m * k, 16)), _ptr(cand_act, torch.int64, "cand_act", dev, (m, k)),
+        _ptr(cand_count, torch.int32, "cand_count", dev, (m,)), _stream())
+    _check(rc, "narde_segment_topk")
+
+
+def lookahead_expand(cand_lo, cand_hi, cand_count, lo, hi, dice):
+    """narde_lookahead_expand: the P = n * k * 21 reply positions (lo / hi [P, 16], dice [P, 2]) of the candidates
+    (cand_lo / cand_hi [n * k, 16], cand_count [n])."""
+    import torch
+
+    dev, n = _device(), cand_count.shape[0]
+    k = cand_lo.shape[0] // n if n else 0
+    if n == 0 or cand_lo.shape[0] != n * k or not 1 <= k <= LOOKAHEAD_MAX_CANDIDATES:
+        raise NardeCudaError("cand_lo must have n * k rows, 1 <= k <= %d" % LOOKAHEAD_MAX_CANDIDATES)
+    p = n * k * LOOKAHEAD_ROLLS
+    rc = load().narde_lookahead_expand(
+        _ptr(cand_lo, torch.uint8, "cand_lo", dev, (n * k, 16)), _ptr(cand_hi, torch.uint8, "cand_hi", dev, (n * k, 16)),
+        _ptr(cand_count, torch.int32, "cand_count", dev, (n,)), n, k, _ptr(lo, torch.uint8, "lo", dev, (p, 16)),
+        _ptr(hi, torch.uint8, "hi", dev, (p, 16)), _ptr(dice, torch.uint8, "dice", dev, (p, 2)), _stream())
+    _check(rc, "narde_lookahead_expand")
+
+
+def lookahead_reduce(hi, cand_idx, cand_score, cand_hi, cand_act, cand_count, cap, reply_value, reply_count, reply_eff,
+                     choice, value, act_override=None, cand_value=None, uncovered=None):
+    """narde_lookahead_reduce: the expectimax value of every candidate and the choice per env (include/narde_b200.h)."""
+    import torch
+
+    k = _candidates_k(cand_idx)
+    dev, n = _device(), hi.shape[0]
+    p = n * k * LOOKAHEAD_ROLLS
+    rc = load().narde_lookahead_reduce(
+        _ptr(hi, torch.uint8, "hi", dev, (n, 16)), _ptr(cand_idx, torch.int32, "cand_idx", dev, (n, k)),
+        _ptr(cand_score, torch.float32, "cand_score", dev, (n, k)), _ptr(cand_hi, torch.uint8, "cand_hi", dev, (n * k, 16)),
+        _ptr(cand_act, torch.int64, "cand_act", dev, (n, k)), _ptr(cand_count, torch.int32, "cand_count", dev, (n,)), n, k, cap,
+        _ptr(reply_value, torch.float32, "reply_value", dev, (p,)), _ptr(reply_count, torch.int32, "reply_count", dev, (p,)),
+        _ptr(reply_eff, torch.int32, "reply_eff", dev, (p,)), _ptr(choice, torch.int32, "choice", dev, (n,)),
+        _ptr(value, torch.float32, "value", dev, (n,)), _ptr(act_override, torch.int64, "act_override", dev, (n,)),
+        _ptr(cand_value, torch.float32, "cand_value", dev, (n, k)), _ptr(uncovered, torch.int32, "uncovered", dev, (_ANY,), 1),
+        _stream())
+    _check(rc, "narde_lookahead_reduce")
 
 
 def step_chosen(lo, hi, env_base, seed, step, dice, choice, actions, counts, act_override=None, chosen=None, obs198=None,

@@ -38,6 +38,19 @@ class _SideBatch:
         self.value = t.zeros(m, dtype=t.float32, device=dev)
 
 
+def _score_side_batch(mlp, sb, lo, hi, dice, overflow, act_override=None, workspace=None):
+    """A side batch up to its scores, on the current stream: gather the positions flagged in `overflow` -> enumerate them
+    with the side capacity (workspace: narde_enumerate_fast's, None = order-dependent turns resolved inline) -> afterstate
+    rows (bounded by sb.rows_cap) -> score."""
+    _cabi.gather_overflow(lo, hi, dice, overflow, sb.lo, sb.hi, sb.dice, sb.idx, sb.ctrl, act_override=act_override)
+    _cabi.enumerate_actions_fast(sb.lo, sb.hi, sb.dice, sb.actions, sb.counts, sb.ovf, workspace)
+    _cabi.afterstates_scan(sb.lo, sb.hi, sb.actions, sb.counts, sb.as_lo, sb.as_hi, sb.scan_ws, offsets=sb.offsets,
+                           rows_out=sb.rows_dev, rows_cap=sb.rows_cap, counts_eff=sb.counts_eff)
+    # (the scorer keeps no state between launches, so this one may be queued beside the first pass's: its CTAs get their
+    # SMs when those leave)
+    mlp.score_states(sb.as_lo, sb.as_hi, out=sb.scores, rows_dev=sb.rows_dev)
+
+
 class AfterstateActor:
     def __init__(self, env, mlp, mode="max", overflow_slots=None, overflow_cap=3072, overflow_rows=None, epsilon=0.0,
                  temperature=0.0):
@@ -145,14 +158,8 @@ class AfterstateActor:
             return
         self._s2.wait_stream(t.cuda.current_stream(env.device))
         with t.cuda.stream(self._s2):
-            _cabi.gather_overflow(env.lo, env.hi, self.dice, env.overflow, sb.lo, sb.hi, sb.dice, sb.idx, sb.ctrl,
-                                  act_override=self.act_override)
-            _cabi.enumerate_actions_fast(sb.lo, sb.hi, sb.dice, sb.actions, sb.counts, sb.ovf, sb.ws)
-            _cabi.afterstates_scan(sb.lo, sb.hi, sb.actions, sb.counts, sb.as_lo, sb.as_hi, sb.scan_ws, offsets=sb.offsets,
-                                   rows_out=sb.rows_dev, rows_cap=sb.rows_cap, counts_eff=sb.counts_eff)
-            # (the scorer keeps no state between launches, so this one may be queued beside the first pass's: its CTAs get
-            # their SMs when those leave)
-            self.mlp.score_states(sb.as_lo, sb.as_hi, out=sb.scores, rows_dev=sb.rows_dev)
+            _score_side_batch(self.mlp, sb, env.lo, env.hi, self.dice, env.overflow, act_override=self.act_override,
+                              workspace=sb.ws)
             # (the same rule over the whole list: the same coin and, per action index, the same noise as the first pass)
             self._segment_choice(sb.scores, sb.offsets, sb.counts_eff, sb.hi, sb.cap, sb.choice, sb.value, step, step_dev,
                                  env_idx=sb.idx)

@@ -17,6 +17,7 @@ namespace narde { __device__ int g_dbg_flags = 0; }
 #include "narde_block.cuh"
 #include "narde_deferred.cuh"
 #include "narde_env.cuh"
+#include "narde_lookahead.cuh"
 
 using namespace narde;
 
@@ -989,6 +990,183 @@ __global__ void __launch_bounds__(kThreads) k_segment_argmax(const float* score,
   if (best_out) best_out[i] = g.c ? (kSample ? score[g.base + best_k] : g.sign * best) : 0.0f;
 }
 
+// Candidates of the one-ply lookahead (narde_segment_topk): the first K entries of each segment in the order of the
+// choice rule (la_before), with their scores, afterstate rows and action words.  Slot i writes to env env_idx[i] when a
+// side batch's env_idx is given (-1: an unused slot), else to env i.
+struct TopkArgs {
+  const float* score;
+  const int64_t* offsets;
+  const int32_t* counts;
+  const uint4* hi;
+  int64_t n;
+  int cap, mode, K;
+  const uint4* as_lo;
+  const uint4* as_hi;
+  const uint64_t* actions;  // [n, cap]
+  const int32_t* env_idx;
+  const int32_t* counts_eff;
+  int32_t* ctrl;
+  int32_t* cand_idx;
+  float* cand_score;
+  uint4* cand_lo;
+  uint4* cand_hi;
+  uint64_t* cand_act;
+  int32_t* cand_count;
+};
+// The slot's env (-1: skip it) and its segment, with the side batch's accounting of narde_scatter_choice: a slot whose
+// rows did not fit (counts_eff 0) is skipped and, like one whose list exceeds cap, counted in *missed.
+__device__ __forceinline__ int64_t topk_begin(const TopkArgs& A, int64_t i, int* c, int64_t* base, float* sign, int* missed) {
+  int64_t e = i;
+  if (A.env_idx) {
+    e = A.env_idx[i];
+    if (e < 0) return -1;
+    if (A.counts_eff && A.counts_eff[i] == 0) {
+      (*missed)++;
+      return -1;
+    }
+    if (A.counts[i] > A.cap) (*missed)++;
+  }
+  const int cnt = A.counts[i];
+  *c = cnt < A.cap ? cnt : A.cap;
+  *base = A.offsets[i];
+  *sign = (A.mode == 1 && (int)(int8_t)((A.hi[i].z >> 16) & 0xFF) != 1) ? -1.0f : 1.0f;
+  return e;
+}
+__device__ __forceinline__ void topk_store(const TopkArgs& A, int64_t i, int64_t e, int64_t base, int j, int k) {
+  const int64_t o = e * A.K + j;
+  A.cand_idx[o] = k;
+  A.cand_score[o] = A.score[base + k];
+  A.cand_lo[o] = A.as_lo[base + k];
+  A.cand_hi[o] = A.as_hi[base + k];
+  A.cand_act[o] = A.actions[i * A.cap + k];
+}
+__device__ __forceinline__ void topk_account(const TopkArgs& A, int missed) {
+  if (!A.ctrl) return;
+  if (missed) atomicAdd(&A.ctrl[2], missed);
+  if (blockIdx.x == 0 && threadIdx.x == 0) A.ctrl[0] = 0;  // ready for the next gather, as narde_scatter_choice leaves it
+}
+
+// A thread per segment (cap <= 128): la_topk over the segment.
+__global__ void __launch_bounds__(kThreads) k_segment_topk(TopkArgs A) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int missed = 0;
+  if (i < A.n) {
+    int c;
+    int64_t base;
+    float sign;
+    const int64_t e = topk_begin(A, i, &c, &base, &sign, &missed);
+    if (e >= 0) {
+      int32_t idx[kLookaheadMaxCandidates];
+      const int got = la_topk(A.score + base, c, sign, A.K, idx);
+      for (int j = 0; j < got; j++) topk_store(A, i, e, base, j, idx[j]);
+      A.cand_count[e] = got;
+    }
+  }
+  topk_account(A, missed);
+}
+
+// A warp per segment (long lists): round j finds the j-th entry -- each lane scans its stride for the first entry after
+// the previous round's, a butterfly of shuffles leaves the first of the lanes' in every lane -- and lane j stores it.
+__global__ void __launch_bounds__(kThreads) k_segment_topk_warp(TopkArgs A) {
+  const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  int missed = 0;
+  if (i < A.n) {  // (whole warps take the same branches)
+    int c;
+    int64_t base;
+    float sign;
+    const int64_t e = topk_begin(A, i, &c, &base, &sign, &missed);
+    if (e >= 0) {
+      bool has = false;
+      float pv = 0.0f;
+      int pk = 0, got = 0, mine = -1;
+      for (; got < A.K; got++) {
+        float v;
+        int k = la_topk_scan(A.score + base, c, sign, has, pv, pk, lane, 32, &v);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          const float ov = __shfl_xor_sync(0xFFFFFFFFu, v, o);
+          const int ok = __shfl_xor_sync(0xFFFFFFFFu, k, o);
+          if (ok >= 0 && (k < 0 || la_before(ov, ok, v, k))) {
+            v = ov;
+            k = ok;
+          }
+        }
+        if (k < 0) break;
+        if (lane == got) mine = k;
+        has = true;
+        pv = v;
+        pk = k;
+      }
+      if (mine >= 0) topk_store(A, i, e, base, lane, mine);
+      if (lane == 0) A.cand_count[e] = got;
+    }
+  }
+  topk_account(A, lane == 0 ? missed : 0);  // (every lane of the warp counted the same slot)
+}
+
+// The reply positions of the lookahead: position p = (i * K + j) * 21 + d is candidate j of env i with roll d of the
+// table; a slot j >= cand_count[i] becomes a finished game (no legal action).
+__global__ void __launch_bounds__(kThreads) k_lookahead_expand(const uint4* cand_lo, const uint4* cand_hi, const int32_t* cand_count,
+                                                              int64_t n, int K, uint4* lo, uint4* hi, uint8_t* dice) {
+  const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n * K * kLookaheadRolls) return;
+  const int64_t slot = p / kLookaheadRolls;
+  const int d = (int)(p - slot * kLookaheadRolls);
+  const int64_t i = slot / K;
+  const int j = (int)(slot - i * K);
+  if (j < cand_count[i]) {
+    lo[p] = cand_lo[slot];
+    hi[p] = cand_hi[slot];
+  } else {
+    State fin;
+    for (int k = 0; k < 6; k++) fin.w[k] = 0;
+    fin.set_meta(15, 0, 1, FLAG_DONE);
+    fin.aux = 0;
+    st_state(lo, hi, p, fin);
+  }
+  int a, b;
+  la_roll(d, &a, &b);
+  reinterpret_cast<uint16_t*>(dice)[p] = (uint16_t)(a | (b << 8));
+}
+
+// Value per candidate (la_candidate_value) and the choice among them (la_pick), a thread per env.  The env's side to
+// move gives the sign: the net scores for WHITE, WHITE maximises.
+__global__ void __launch_bounds__(kThreads) k_lookahead_reduce(const uint4* hi, const int32_t* cand_idx, const float* cand_score,
+                                                              const uint4* cand_hi, const uint64_t* cand_act,
+                                                              const int32_t* cand_count, int64_t n, int K, int cap,
+                                                              const float* reply_value, const int32_t* reply_count,
+                                                              const int32_t* reply_eff, int32_t* choice, float* value,
+                                                              uint64_t* act_override, float* cand_value, int32_t* uncovered) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int cnt = cand_count[i];
+  const float sign = (int)(int8_t)((hi[i].z >> 16) & 0xFF) == 1 ? 1.0f : -1.0f;
+  float v[kLookaheadMaxCandidates];
+  bool any_unfit = false;
+  for (int j = 0; j < cnt; j++) {
+    const int64_t slot = i * K + j;
+    const int64_t p = slot * kLookaheadRolls;
+    const bool terminal = ((cand_hi[slot].z >> 24) & FLAG_DONE) != 0;
+    bool unfit;
+    v[j] = la_candidate_value(cand_score[slot], terminal, reply_value + p, reply_count + p, reply_eff + p, &unfit);
+    any_unfit |= unfit;
+    if (cand_value) cand_value[slot] = v[j];
+  }
+  if (cnt == 0) {
+    choice[i] = 0;
+    value[i] = 0.0f;
+    if (act_override) act_override[i] = 0ull;
+  } else {
+    const int best = la_pick(v, cnt, sign);
+    const int k = cand_idx[i * K + best];
+    choice[i] = k;
+    value[i] = v[best];
+    if (act_override) act_override[i] = k >= cap ? cand_act[i * K + best] : 0ull;
+  }
+  if (any_unfit && uncovered) atomicAdd(uncovered, 1);
+}
+
 // Trainer-compatible action codes (train_deepq_pytorch.py:432-437,495-507,752-761): for every stored legal
 // turn action the reference's (move1_code, move2_code) pair, code = from*24 + to with to = 0 for a bear-off
 // and move2_code = 0 when the turn has one half-move.  Only the first two half-moves are representable in
@@ -1369,6 +1547,52 @@ int narde_segment_sample(const float* score, const int64_t* offsets, const int32
   if (n < 0 || cap <= 0 || !score || !offsets || !counts || !hi || !params || !idx_out || !aligned16(hi)) return -1;
   const SampleArgs S = {params, env_idx, env_base, seed, step, step_dev};
   return launch_segment<true>(score, offsets, counts, hi, n, cap, mode, idx_out, value_out, S, stream);
+}
+
+int narde_segment_topk(const float* score, const int64_t* offsets, const int32_t* counts, const void* hi, int64_t n, int32_t cap,
+                       int32_t mode, int32_t k, const void* as_lo, const void* as_hi, const uint64_t* actions,
+                       const int32_t* env_idx, const int32_t* counts_eff, int32_t* ctrl, int32_t* cand_idx, float* cand_score,
+                       void* cand_lo, void* cand_hi, uint64_t* cand_act, int32_t* cand_count, void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || cap <= 0 || k < 1 || k > NARDE_LOOKAHEAD_MAX_CANDIDATES || (mode != 0 && mode != 1)) return -1;
+  if (!score || !offsets || !counts || !hi || !as_lo || !as_hi || !actions || !cand_idx || !cand_score || !cand_lo ||
+      !cand_hi || !cand_act || !cand_count)
+    return -1;
+  if (!aligned16(hi) || !aligned16(as_lo) || !aligned16(as_hi) || !aligned16(cand_lo) || !aligned16(cand_hi)) return -1;
+  const TopkArgs A = {score, offsets, counts, (const uint4*)hi, n, cap, mode, k, (const uint4*)as_lo, (const uint4*)as_hi,
+                      actions, env_idx, counts_eff, ctrl, cand_idx, cand_score, (uint4*)cand_lo, (uint4*)cand_hi, cand_act,
+                      cand_count};
+  if (cap > 128)  // long segments: a warp per env, as launch_segment
+    k_segment_topk_warp<<<grid_for(n * 32), kThreads, 0, (cudaStream_t)stream>>>(A);
+  else
+    k_segment_topk<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>(A);
+  return launch_status();
+}
+
+int narde_lookahead_expand(const void* cand_lo, const void* cand_hi, const int32_t* cand_count, int64_t n, int32_t k, void* lo,
+                           void* hi, uint8_t* dice, void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || k < 1 || k > NARDE_LOOKAHEAD_MAX_CANDIDATES || !cand_lo || !cand_hi || !cand_count || !lo || !hi || !dice) return -1;
+  if (!aligned16(cand_lo) || !aligned16(cand_hi) || !aligned16(lo) || !aligned16(hi) || (((uintptr_t)dice) & 1u) != 0) return -1;
+  k_lookahead_expand<<<grid_for(n * k * kLookaheadRolls), kThreads, 0, (cudaStream_t)stream>>>(
+      (const uint4*)cand_lo, (const uint4*)cand_hi, cand_count, n, k, (uint4*)lo, (uint4*)hi, dice);
+  return launch_status();
+}
+
+int narde_lookahead_reduce(const void* hi, const int32_t* cand_idx, const float* cand_score, const void* cand_hi,
+                           const uint64_t* cand_act, const int32_t* cand_count, int64_t n, int32_t k, int32_t cap,
+                           const float* reply_value, const int32_t* reply_count, const int32_t* reply_eff, int32_t* choice,
+                           float* value, uint64_t* act_override, float* cand_value, int32_t* uncovered, void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || k < 1 || k > NARDE_LOOKAHEAD_MAX_CANDIDATES || cap <= 0) return -1;
+  if (!hi || !cand_idx || !cand_score || !cand_hi || !cand_act || !cand_count || !reply_value || !reply_count || !reply_eff ||
+      !choice || !value)
+    return -1;
+  if (!aligned16(hi) || !aligned16(cand_hi)) return -1;
+  k_lookahead_reduce<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>(
+      (const uint4*)hi, cand_idx, cand_score, (const uint4*)cand_hi, cand_act, cand_count, n, k, cap, reply_value, reply_count,
+      reply_eff, choice, value, act_override, cand_value, uncovered);
+  return launch_status();
 }
 
 int narde_action_codes(const uint64_t* actions, const int32_t* counts, int64_t n, int32_t cap, int32_t* codes, void* stream) {

@@ -305,6 +305,58 @@ int narde_segment_sample(const float *score, const int64_t *offsets, const int32
                          uint64_t seed, uint64_t step, const uint64_t *step_dev, const float *params,
                          int32_t *idx_out, float *value_out, void *stream);
 
+/* One-ply expectimax lookahead (gym_narde_b200.LookaheadActor), for a net that scores positions for WHITE (mode 1 above:
+ * WHITE maximises, BLACK minimises).  Per env turn, with s0[a] the 0-ply score of legal action a and sign = +1 when WHITE
+ * is to move, -1 otherwise:
+ *   1. candidates: the first K = min(candidates, count) actions of the whole legal list in the order of the choice rule of
+ *      narde_segment_argmax over sign * s0 (larger first, ties to the lower index, a NaN after every number): slot 0 is
+ *      the greedy choice;
+ *   2. replies: for candidate afterstate c and roll d of the fixed table 1-1, 1-2, ..., 1-6, 2-2, ..., 6-6 (21 rolls,
+ *      weight w_d = 1 for doubles, 2 otherwise: 36 in all), r[c,d] = the opponent's best reply score, narde_segment_argmax
+ *      mode 1 over the full legal list of c with dice d; r[c,d] = s0[c] when the opponent has no legal move;
+ *   3. value: v[c] = acc / 36.0f, acc summed in float32 in roll order, acc += w_d * r[c,d]; v[c] = s0[c] when the
+ *      afterstate c ends the game; v[c] = NaN when some roll's reply list was not scored in full (row pool or side batch
+ *      too small);
+ *   4. choice: the candidate with the largest sign * v (ties to the lower slot, a NaN never wins; all NaN: slot 0).
+ * With K = 1 the action is the greedy one of narde_segment_argmax, bit for bit. */
+#define NARDE_LOOKAHEAD_ROLLS 21
+#define NARDE_LOOKAHEAD_MAX_CANDIDATES 32
+
+/* Step 1 over the segments of narde_segment_argmax (same score / offsets / counts / hi / cap / mode): for each env, up to
+ * k <= NARDE_LOOKAHEAD_MAX_CANDIDATES candidates in slot order -- cand_idx [.., k] i32 the action index, cand_score
+ * [.., k] f32 its score, cand_lo / cand_hi [.. * k] 16-byte lanes its afterstate row (as_lo / as_hi at offsets[i] + index),
+ * cand_act [.., k] u64 its action word (actions [n, cap], row i) -- and cand_count [..] = min(k, min(counts[i], cap)); slots
+ * at or beyond cand_count are not written.  A thread per env for cap <= 128, a warp per env above.
+ * env_idx (may be NULL): slot i writes env env_idx[i]'s candidates instead of its own, -1 = unused slot -- the side
+ * batch of narde_gather_overflow overwriting the candidates of the envs it covers; then, as narde_scatter_choice does, a
+ * slot with counts_eff[i] == 0 (counts_eff may be NULL) is skipped, it and a slot with counts[i] > cap add one to
+ * ctrl[2], and ctrl[0] is cleared (ctrl may be NULL). */
+int narde_segment_topk(const float *score, const int64_t *offsets, const int32_t *counts, const void *hi, int64_t n,
+                       int32_t cap, int32_t mode, int32_t k, const void *as_lo, const void *as_hi, const uint64_t *actions,
+                       const int32_t *env_idx, const int32_t *counts_eff, int32_t *ctrl, int32_t *cand_idx,
+                       float *cand_score, void *cand_lo, void *cand_hi, uint64_t *cand_act, int32_t *cand_count,
+                       void *stream);
+
+/* The P = n * k * NARDE_LOOKAHEAD_ROLLS reply positions of step 2: position (i * k + j) * 21 + d is candidate j of env i
+ * (cand_lo / cand_hi as narde_segment_topk writes them) with dice (a, b) = roll d of the table; a slot j >=
+ * cand_count[i] becomes a finished game (no legal action).  lo / hi [P] 16-byte lanes, dice [P, 2] u8. */
+int narde_lookahead_expand(const void *cand_lo, const void *cand_hi, const int32_t *cand_count, int64_t n, int32_t k,
+                           void *lo, void *hi, uint8_t *dice, void *stream);
+
+/* Steps 3 and 4 from the reply positions' results: reply_value [P] the best-reply score (narde_segment_argmax mode 1
+ * best_out), reply_count [P] the legal count (0: blocked), reply_eff [P] the length of the list prefix the reply was
+ * chosen from (reply_eff < reply_count: not scored in full, e.g. 0 when its rows did not fit the row pool); a terminal
+ * candidate has the done flag in cand_hi.  hi: the envs' states (side to move).  Writes choice [n] i32 = cand_idx of the
+ * chosen slot, value [n] f32 = its v, act_override [n] u64 (may be NULL) = its action word when the index is >= cap
+ * (beyond the stored lists of narde_step_chosen), else 0, cand_value [n, k] f32 (may be NULL) = v of every candidate, and
+ * adds to *uncovered (may be NULL) the number of envs with a NaN candidate from step 3.  An env without candidates gets
+ * choice 0, value 0. */
+int narde_lookahead_reduce(const void *hi, const int32_t *cand_idx, const float *cand_score, const void *cand_hi,
+                           const uint64_t *cand_act, const int32_t *cand_count, int64_t n, int32_t k, int32_t cap,
+                           const float *reply_value, const int32_t *reply_count, const int32_t *reply_eff,
+                           int32_t *choice, float *value, uint64_t *act_override, float *cand_value,
+                           int32_t *uncovered, void *stream);
+
 /* Trainer-compatible action codes for every stored legal turn action: the reference's (move1_code,
  * move2_code) pairs (train_deepq_pytorch.py:432-437,495-507; action_to_idx :752-761): code = from*24 + to,
  * to = 0 for a bear-off, move2_code = 0 when the turn has a single half-move.  codes: [n,cap,3] i32 =
