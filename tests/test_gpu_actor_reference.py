@@ -434,10 +434,12 @@ class _Turn:
         return ref_choice(sc, np.minimum(self.counts, prefix), self.sign, cap)
 
 
-def _actor(design, cap, mode, n=3001, max_episode_steps=90, **kw):
+def _actor(design, cap, mode, n=3001, max_episode_steps=90, seed=None, env_base=0, **kw):
+    """env and actor after 60 random turns; seed None: 1234 + cap.  kw: the actor's pools (none: its defaults)."""
     from gym_narde_b200 import VecNardeEnv, AfterstateMLP, AfterstateActor
     W, b = design
-    env = VecNardeEnv(n, seed=1234 + cap, max_actions=cap, max_episode_steps=max_episode_steps)
+    env = VecNardeEnv(n, seed=1234 + cap if seed is None else seed, max_actions=cap, max_episode_steps=max_episode_steps,
+                      env_base=env_base)
     mlp = AfterstateMLP(W[0], b[0], W[1], b[1], W[2], b[2])
     actor = AfterstateActor(env, mlp, mode=mode, **kw)
     env.reset()
@@ -450,6 +452,54 @@ def _play(env, actor, graph):
     lo, hi = env.lo.cpu().numpy(), env.hi.cpu().numpy()
     actor.step_graph() if graph else actor.step()
     return lo, hi, actor.dice.cpu().numpy()
+
+
+def check_exact_turn(ref, choice, value, chosen, what):
+    """The exact-scorer rule of one turn: every live env's choice is ref_choice over the oracle's full list, value is its
+    reference score bit for bit, the action played is the oracle's action at that index; envs without an action have
+    (0, 0).  Returns the live env indices and the reference's choices."""
+    want_k, want_v = ref.choice()
+    live = ref.counts > 0
+    bad = np.flatnonzero(live & (choice != want_k))
+    assert len(bad) == 0, ("choice", what, len(bad), [(int(i), int(ref.counts[i]), int(choice[i]), int(want_k[i]))
+                                                      for i in bad[:5]])
+    assert same_floats(value[live], want_v[live]), ("value", what)
+    assert (choice[~live] == 0).all() and (value[~live] == 0).all(), what
+    rows = np.flatnonzero(live)
+    assert np.array_equal(chosen[rows], ref.acts[rows, want_k[rows]]), ("action", what)
+    return rows, want_k
+
+
+def check_within_bound(ref, choice, value, what):
+    """The realistic-scorer rule of one turn (ref: a _Turn with_bound), over every live env at once: where the best plain
+    float64 score beats the second by more than twice the env's largest bound(), the choice is the reference's; elsewhere
+    the chosen action's score is within 2 * bound of the best; value is within bound() of the plain score of the chosen
+    row.  Returns (env turns decided by more than 2 bound, near-ties)."""
+    n = len(choice)
+    rows = np.arange(n)
+    live = ref.counts > 0
+    signed = np.where(ref.mask, ref.q * ref.sign[:, None], -np.inf)
+    top = signed.argmax(1)                                   # the first index of the maximum
+    best = signed[rows, top]
+    rest = signed.copy()
+    rest[rows, top] = -np.inf
+    second = rest.max(1)
+    lim = np.where(ref.mask, ref.bnd, 0).max(1)
+    with np.errstate(invalid="ignore"):                      # (envs without an action: -inf - -inf)
+        clear = best - second > 2 * lim
+    k = choice.astype(np.int64)
+    inside = (k >= 0) & (k < ref.counts)
+    assert inside[live].all(), ("index", what, np.flatnonzero(live & ~inside)[:5])
+    k = np.where(live, k, 0)
+    ok = np.where(clear, k == top, signed[rows, k] >= best - 2 * lim)
+    bad = np.flatnonzero(live & ~ok)
+    assert len(bad) == 0, ("choice", what, len(bad), [(int(i), int(k[i]), int(top[i]), best[i] - second[i], lim[i])
+                                                      for i in bad[:5]])
+    err = np.abs(value.astype(np.float64) - ref.q[rows, k])
+    bad = np.flatnonzero(live & ~(err <= ref.bnd[rows, k]))           # (a NaN value fails)
+    assert len(bad) == 0, ("value", what, len(bad), [(int(i), float(value[i]), ref.q[i, k[i]], ref.bnd[i, k[i]])
+                                                     for i in bad[:5]])
+    return int((clear & live).sum()), int((~clear & live).sum())
 
 
 EXACT_RUNS = [("perm", 64, "max", False), ("sparse", 64, "white_value", True), ("argmax", 8, "white_value", False),
@@ -471,17 +521,9 @@ def test_actor_plays_the_reference_choice_with_an_exact_scorer(design, cap, mode
         lo, hi, dice = _play(env, actor, graph)
         ref = _Turn(lo, hi, dice, env.counts, W, b, m, emulate=True, premise=(t % 25 == 0))
         choice, value, chosen = actor.choice.cpu().numpy(), actor.value.cpu().numpy(), env.chosen.cpu().numpy()
-        want_k, want_v = ref.choice()
-        live = ref.counts > 0
-        bad = np.flatnonzero(live & (choice != want_k))
-        assert len(bad) == 0, ("choice", design, cap, mode, t, len(bad), [(int(i), int(ref.counts[i]), int(choice[i]),
-                                                                           int(want_k[i])) for i in bad[:5]])
-        assert same_floats(value[live], want_v[live]), ("value", design, cap, mode, t)
-        assert (choice[~live] == 0).all() and (value[~live] == 0).all(), t
-        rows = np.flatnonzero(live)
-        assert np.array_equal(chosen[rows], ref.acts[rows, want_k[rows]]), ("action", t)
+        rows, want_k = check_exact_turn(ref, choice, value, chosen, (design, cap, mode, t))
         checked += len(rows)
-        beyond += int((want_k[live] >= cap).sum())
+        beyond += int((want_k[rows] >= cap).sum())
         ends += int((env.done.cpu().numpy() != 0).sum())
         truncs += int((env.trunc.cpu().numpy() != 0).sum())
         half = (chosen[rows].astype(np.uint64)[:, None] >> np.arange(0, 64, 16, dtype=np.uint64)) & np.uint64(0xFFFF)
@@ -508,25 +550,9 @@ def test_actor_with_a_realistic_scorer_is_within_the_bound(scale):
         for t in range(25):
             lo, hi, dice = _play(env, actor, False)
             ref = _Turn(lo, hi, dice, env.counts, W, b, 1 if mode == "white_value" else 0, emulate=False, with_bound=True)
-            choice, value = actor.choice.cpu().numpy(), actor.value.cpu().numpy().astype(np.float64)
-            live = np.flatnonzero(ref.counts > 0)
-            signed = np.where(ref.mask, ref.q * ref.sign[:, None], -np.inf)
-            order = np.argsort(-signed, axis=1, kind="stable")
-            best = signed[np.arange(len(signed)), order[:, 0]]
-            second = np.where(ref.counts > 1, signed[np.arange(len(signed)), order[:, min(1, signed.shape[1] - 1)]],
-                              -np.inf)
-            lim = np.where(ref.mask, ref.bnd, 0).max(1)
-            clear = best - second > 2 * lim
-            for i in live:
-                k = choice[i]
-                assert 0 <= k < ref.counts[i], (mode, t, i)
-                if clear[i]:
-                    assert k == order[i, 0], (mode, t, i, k, order[i, 0], best[i] - second[i], lim[i])
-                else:
-                    assert signed[i, k] >= best[i] - 2 * lim[i], (mode, t, i)
-                assert abs(value[i] - ref.q[i, k]) <= ref.bnd[i, k], (mode, t, i, value[i], ref.q[i, k], ref.bnd[i, k])
-            decided += int(clear[live].sum())
-            near += int((~clear[live]).sum())
+            d, e = check_within_bound(ref, actor.choice.cpu().numpy(), actor.value.cpu().numpy(), (mode, t))
+            decided += d
+            near += e
         assert actor.uncovered_envs() == 0
     share = near / max(1, decided + near)
     print("realistic x%g: %d env turns decided by more than 2 bound, %d near-ties (%.4f)" % (scale, decided, near, share))

@@ -489,6 +489,23 @@ def _sign(hi):
     return np.where(hi[:, 10].view(np.int8) == 1, 1.0, -1.0).astype(np.float32)
 
 
+def _best_replies(lo, hi, dice, W, b, emulate, with_bound, chunk=1 << 16):
+    """The opponent's side of every reply position, `chunk` positions at a time (so _scored's [positions, longest list]
+    arrays stay small at millions of positions): (legal counts [p], the score of the choice over the whole list
+    float32 [p], the largest bound() of its rows [p] or None)."""
+    p = len(lo)
+    rc, best = np.zeros(p, np.int32), np.zeros(p, np.float32)
+    rb = np.zeros(p) if with_bound else None
+    for s in range(0, p, chunk):
+        e = min(s + chunk, p)
+        c, _, _, _, q, bd = _scored(lo[s:e], hi[s:e], dice[s:e], W, b, emulate, with_bound)
+        rc[s:e] = c
+        best[s:e] = ref_choice(q.astype(np.float32), c, _sign(hi[s:e]), q.shape[1])[1]
+        if with_bound:
+            rb[s:e] = np.where(np.arange(bd.shape[1])[None, :] < c[:, None], bd, 0).max(1)
+    return rc, best, rb
+
+
 class _LookTurn:
     """The reference of one lookahead turn from the positions before it: the first pass over the oracle's full lists, the
     top-K, the oracle's full reply lists of every (candidate, roll), each scored by the float64 net, and the numpy rule.
@@ -508,8 +525,8 @@ class _LookTurn:
         c_lo, c_hi = a_lo[ii, kk], a_hi[ii, kk]
         p_lo, p_hi = np.repeat(c_lo, 21, 0), np.repeat(c_hi, 21, 0)
         p_dice = np.tile(np.array(ROLLS, np.uint8), (len(ii), 1))
-        rc, _, r_lo, r_hi, r_q, r_b = _scored(p_lo, p_hi, p_dice, W, b, emulate, with_bound)
-        r_best = ref_choice(r_q.astype(np.float32), rc, _sign(p_hi), r_q.shape[1])[1]
+        rc, r_best, rb = _best_replies(p_lo, p_hi, p_dice, W, b, emulate, with_bound)
+        self.reply_rows = int(rc.sum())
         self.terminal = np.zeros((n, K), bool)
         self.terminal[ii, jj] = (c_hi[:, 11] & 4) != 0
         self.r_counts = np.zeros((n, K, 21), np.int32)
@@ -528,18 +545,20 @@ class _LookTurn:
         self.live_slots = live
         if with_bound:
             b_env = np.where(self.counts[:, None] > np.arange(self.bnd.shape[1])[None, :], self.bnd, 0).max(1)
-            rb = np.where(np.arange(r_b.shape[1])[None, :] < rc[:, None], r_b, 0).max(1)
             per = np.zeros(n)
             np.maximum.at(per, np.repeat(ii, 21), rb)
             self.B = np.maximum(b_env, per)
 
 
-def _lookahead(design, K, cap, reply_cap, n=512, seed=77, **kw):
+def _lookahead(design, K, cap, reply_cap, n=512, seed=None, env_base=0, slot_per_env=True, **kw):
+    """env and actor after 60 random turns; seed None: 77 + cap + K.  slot_per_env: a first-pass side batch slot for
+    every env unless kw sets overflow_slots (False: the actor's default pools, as far as kw leaves them)."""
     from gym_narde_b200 import AfterstateMLP, LookaheadActor, VecNardeEnv
     W, b = design
-    env = VecNardeEnv(n, seed=seed + cap + K, max_actions=cap)
+    env = VecNardeEnv(n, seed=77 + cap + K if seed is None else seed, max_actions=cap, env_base=env_base)
     mlp = AfterstateMLP(W[0], b[0], W[1], b[1], W[2], b[2])
-    kw.setdefault("overflow_slots", n)
+    if slot_per_env:
+        kw.setdefault("overflow_slots", n)
     actor = LookaheadActor(env, mlp, candidates=K, reply_cap=reply_cap, **kw)
     env.reset()
     for _ in range(60):                       # random self-play: positions of every phase
@@ -551,6 +570,56 @@ def _play(env, actor, graph):
     lo, hi = env.lo.cpu().numpy(), env.hi.cpu().numpy()
     actor.step_graph() if graph else actor.step()
     return lo, hi, actor.dice.cpu().numpy()
+
+
+def check_look_turn(ref, env, actor, cap, reply_cap, seen, what):
+    """The exact-scorer rule of one lookahead turn: choice, value and the action played equal the reference bit for bit
+    for every env.  Adds to `seen` what the turn crossed: live env turns, blocked replies, terminal candidates, reply
+    lists longer than reply_cap, candidates beyond the stored list, envs where lookahead played another action than
+    greedy."""
+    choice, value, chosen = actor.choice.cpu().numpy(), actor.value.cpu().numpy(), env.chosen.cpu().numpy()
+    live = ref.counts > 0
+    bad = np.flatnonzero(choice != ref.choice)
+    assert len(bad) == 0, ("choice", what, len(bad),
+                           [(int(i), int(ref.counts[i]), int(choice[i]), int(ref.choice[i])) for i in bad[:5]])
+    assert same_floats(value, ref.value), ("value", what,
+                                           np.flatnonzero(value.view(np.int32) != ref.value.view(np.int32))[:5])
+    rows = np.flatnonzero(live)
+    assert np.array_equal(chosen[rows], ref.acts[rows, ref.choice[rows]]), ("action", what)
+    ls = ref.live_slots
+    seen["turns"] += int(live.sum())
+    seen["blocked"] += int(((ref.r_counts == 0) & (ls & ~ref.terminal)[:, :, None]).sum())
+    seen["terminal"] += int((ref.terminal & ls).sum())
+    seen["reply_side"] += int(((ref.r_counts > reply_cap) & ls[:, :, None]).sum())
+    seen["beyond"] += int(((ref.idx >= cap) & ls).sum())
+    seen["differ"] += int((live & (ref.choice != ref.idx[:, 0])).sum())
+
+
+def check_look_bound(ref, actor, K, what):
+    """The realistic-scorer rule of one lookahead turn (ref: a _LookTurn with_bound over the actor's own candidates),
+    B = the largest bound() over an env's first-pass and reply rows: the candidates are within 2B of the reference's K-th
+    best 0-ply score; where the reference's best and second-best v differ by more than 2B the actor plays the reference's
+    best, elsewhere an action whose reference v is within 2B of the best.  Returns (decided, near-ties)."""
+    c_idx, c_cnt = actor.cand_idx.cpu().numpy(), actor.cand_count.cpu().numpy()
+    choice = actor.choice.cpu().numpy()
+    decided = near = 0
+    for i in np.flatnonzero(ref.counts > 0):
+        B = ref.B[i]
+        g = int(c_cnt[i])
+        assert g == min(K, ref.counts[i]), (what, i)
+        signed0 = ref.sign[i] * ref.q[i, :ref.counts[i]]
+        kth_best = np.sort(signed0)[::-1][g - 1]
+        assert (ref.sign[i] * ref.q[i, c_idx[i, :g]] >= kth_best - 2 * B).all(), (what, i)
+        sv = ref.sign[i] * ref.v[i, :g].astype(np.float64)
+        order = np.argsort(-sv, kind="stable")
+        slot = int(np.flatnonzero(c_idx[i, :g] == choice[i])[0])
+        if g > 1 and sv[order[0]] - sv[order[1]] > 2 * B:
+            assert slot == order[0], (what, i, slot, order[0], sv, B)
+            decided += 1
+        else:
+            assert sv[slot] >= sv[order[0]] - 2 * B, (what, i)
+            near += 1
+    return decided, near
 
 
 EXACT_RUNS = [("perm", 32, 8, 64, True), ("sparse", 4, 64, 8, False), ("argmax", 1, 8, 8, True),
@@ -571,21 +640,7 @@ def test_lookahead_plays_the_reference_with_an_exact_scorer(design, K, cap, repl
     for t in range(30):
         lo, hi, dice = _play(env, actor, graph)
         ref = _LookTurn(lo, hi, dice, K, W, b, premise=(t % 10 == 0))
-        choice, value, chosen = actor.choice.cpu().numpy(), actor.value.cpu().numpy(), env.chosen.cpu().numpy()
-        live = ref.counts > 0
-        bad = np.flatnonzero(choice != ref.choice)
-        assert len(bad) == 0, ("choice", design, K, cap, reply_cap, t, len(bad),
-                               [(int(i), int(ref.counts[i]), int(choice[i]), int(ref.choice[i])) for i in bad[:5]])
-        assert same_floats(value, ref.value), ("value", t, np.flatnonzero(value.view(np.int32) != ref.value.view(np.int32))[:5])
-        rows = np.flatnonzero(live)
-        assert np.array_equal(chosen[rows], ref.acts[rows, ref.choice[rows]]), ("action", t)
-        ls = ref.live_slots
-        seen["turns"] += int(live.sum())
-        seen["blocked"] += int(((ref.r_counts == 0) & (ls & ~ref.terminal)[:, :, None]).sum())
-        seen["terminal"] += int((ref.terminal & ls).sum())
-        seen["reply_side"] += int(((ref.r_counts > reply_cap) & ls[:, :, None]).sum())
-        seen["beyond"] += int(((ref.idx >= cap) & ls).sum())
-        seen["differ"] += int((live & (ref.choice != ref.idx[:, 0])).sum())
+        check_look_turn(ref, env, actor, cap, reply_cap, seen, (design, K, cap, reply_cap, t))
     assert actor.uncovered_envs() == 0
     print("lookahead exact %s K=%d cap %d reply_cap %d %s: %s" % (design, K, cap, reply_cap,
                                                                   "step_graph" if graph else "step", seen))
@@ -634,26 +689,11 @@ def test_lookahead_with_a_realistic_scorer_is_within_the_bound(scale):
     decided = near = 0
     for t in range(8):
         lo, hi, dice = _play(env, actor, False)
-        c_idx, c_cnt = actor.cand_idx.cpu().numpy(), actor.cand_count.cpu().numpy()
-        ref = _LookTurn(lo, hi, dice, K, W, b, emulate=False, with_bound=True, cands=(c_idx, c_cnt))
-        choice = actor.choice.cpu().numpy()
-        kth = ref_topk(ref.s0, ref.counts, ref.sign, K)
-        for i in np.flatnonzero(ref.counts > 0):
-            B = ref.B[i]
-            g = int(c_cnt[i])
-            assert g == min(K, ref.counts[i]), (t, i)
-            signed0 = ref.sign[i] * ref.q[i, :ref.counts[i]]
-            kth_best = np.sort(signed0)[::-1][g - 1]
-            assert (ref.sign[i] * ref.q[i, c_idx[i, :g]] >= kth_best - 2 * B).all(), (t, i)
-            sv = ref.sign[i] * ref.v[i, :g].astype(np.float64)
-            order = np.argsort(-sv, kind="stable")
-            slot = int(np.flatnonzero(c_idx[i, :g] == choice[i])[0])
-            if g > 1 and sv[order[0]] - sv[order[1]] > 2 * B:
-                assert slot == order[0], (t, i, slot, order[0], sv, B)
-                decided += 1
-            else:
-                assert sv[slot] >= sv[order[0]] - 2 * B, (t, i)
-                near += 1
+        cands = (actor.cand_idx.cpu().numpy(), actor.cand_count.cpu().numpy())
+        ref = _LookTurn(lo, hi, dice, K, W, b, emulate=False, with_bound=True, cands=cands)
+        d, e = check_look_bound(ref, actor, K, (scale, t))
+        decided += d
+        near += e
     print("lookahead realistic x%g: %d env turns decided by more than 2B, %d near-ties" % (scale, decided, near))
     assert decided > 20
 
