@@ -5,6 +5,8 @@ Public surface (mirrors gym_narde/__init__.py + gym_narde/envs):
   gym_narde_b200.VecNardeEnv             N lock-step games on the GPU
   gym_narde_b200.AfterstateMLP / AfterstateActor   DecomposedDQN(198) scorer and the greedy batched actor
   gym_narde_b200.LookaheadActor          the same actor with a one-ply expectimax over the opponent's 21 rolls
+  gym_narde_b200.AfterstateMatch         lock-step games of two afterstate nets, or a net and the random agent, tallied
+                                         on the device
   gym_narde_b200.expand_obs198(lo, hi)   packed 32-byte state records -> Box(198) rows (host or device)
   gym_narde_b200.NardeGameManager        interactive turn manager (my_game/narde_game_manager.py surface)
   gym_narde_b200.make(id)                'narde-v0' (reference rules) / 'Narde-v0' (README rules)
@@ -33,6 +35,9 @@ def _lazy(name):
     if name == "LookaheadActor":
         from .lookahead import LookaheadActor
         return LookaheadActor
+    if name == "AfterstateMatch":
+        from .match import AfterstateMatch
+        return AfterstateMatch
     if name == "expand_obs198":
         from .state import expand_obs198
         return expand_obs198

@@ -77,6 +77,10 @@ _SIGNATURES = {
     "narde_lookahead_expand": ([_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp], _int),
     "narde_lookahead_reduce": ([_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
                                _int),
+    "narde_match_split_counts": ([_vp, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _vp], _int),
+    "narde_match_choose": ([_vp, _vp, _i64, _i32, _i64, _vp, _u64, _u64, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
+                            _vp, _vp, _vp, _vp], _int),
+    "narde_match_tally": ([_vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp], _int),
     "narde_obs198": ([_vp, _vp, _i64, _vp, _vp], _int),
     "narde_obs24": ([_vp, _vp, _i64, _vp, _vp], _int),
     "narde_apply_actions": ([_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp], _int),
@@ -487,6 +491,76 @@ def lookahead_reduce(hi, cand_idx, cand_score, cand_hi, cand_act, cand_count, ca
         _ptr(cand_value, torch.float32, "cand_value", dev, (n, k)), _ptr(uncovered, torch.int32, "uncovered", dev, (_ANY,), 1),
         _stream())
     _check(rc, "narde_lookahead_reduce")
+
+
+# -- lock-step matches (gym_narde_b200/match.py) ---------------------------------------------------
+MATCH_TALLIES = 9
+MATCH_TALLY_NAMES = ("games", "a_wins", "b_wins", "a_mars", "b_mars", "truncated", "a_white_wins", "b_white_wins", "plies")
+
+
+def _match_kinds(kinds):
+    if kinds not in (0, 1, 2, 3):
+        raise NardeCudaError("kinds must be in 0..3 (bit 0: seat A is a net, bit 1: seat B), got %r" % (kinds,))
+    return kinds
+
+
+def match_split_counts(hi, counts, env_base, kinds, counts_a=None, counts_b=None, env_idx=None):
+    """narde_match_split_counts: each slot's count goes to counts_a or counts_b ([n] int32), whichever net seat owns the
+    side to move; 0 elsewhere.  The count array of a random seat may be None."""
+    import torch
+
+    dev, n = _device(), hi.shape[0]
+    kinds = _match_kinds(kinds)
+    if (kinds & 1 and counts_a is None) or (kinds & 2 and counts_b is None):
+        raise NardeCudaError("a net seat needs its count array")
+    rc = load().narde_match_split_counts(
+        _ptr(hi, torch.uint8, "hi", dev, (n, 16)), _ptr(counts, torch.int32, "counts", dev, (n,)), n, env_base,
+        _ptr(env_idx, torch.int32, "env_idx", dev, (n,)), kinds, _ptr(counts_a, torch.int32, "counts_a", dev, (n,)),
+        _ptr(counts_b, torch.int32, "counts_b", dev, (n,)), _stream())
+    _check(rc, "narde_match_split_counts")
+
+
+def match_choose(hi, counts, cap, env_base, seed, kinds, modes, pools, choice, value, eff=None, env_idx=None, step=0,
+                 step_dev=None):
+    """narde_match_choose: per slot, the owner's rule on the owner's segment.  modes: (mode_a, mode_b) in {0, 1}; pools:
+    ((score, offsets, counts_eff) or None per seat: None for a random seat)."""
+    import torch
+
+    dev, n = _device(), hi.shape[0]
+    kinds = _match_kinds(kinds)
+    args = []
+    for p in (0, 1):
+        pool = pools[p]
+        if (kinds >> p) & 1:
+            if pool is None:
+                raise NardeCudaError("net seat %d needs its (score, offsets, counts_eff)" % p)
+            if modes[p] not in (0, 1):
+                raise NardeCudaError("mode of seat %d must be 0 or 1, got %r" % (p, modes[p]))
+            sc, off, ce = pool
+            args += [_ptr(sc, torch.float32, "score", dev, (_ANY,)), _ptr(off, torch.int64, "offsets", dev, (n,)),
+                     _ptr(ce, torch.int32, "counts_eff", dev, (n,))]
+        else:
+            args += [None, None, None]
+    rc = load().narde_match_choose(
+        _ptr(hi, torch.uint8, "hi", dev, (n, 16)), _ptr(counts, torch.int32, "counts", dev, (n,)), n, cap, env_base,
+        _ptr(env_idx, torch.int32, "env_idx", dev, (n,)), seed & 0xFFFFFFFFFFFFFFFF, step,
+        _ptr(step_dev, torch.int64, "step_dev", dev, (1,)), kinds, int(modes[0]), int(modes[1]), *args,
+        _ptr(choice, torch.int32, "choice", dev, (n,)), _ptr(value, torch.float32, "value", dev, (n,)),
+        _ptr(eff, torch.int32, "eff", dev, (n,)), _stream())
+    _check(rc, "narde_match_choose")
+
+
+def match_tally(hi, done, truncated, env_base, outcome, tallies):
+    """narde_match_tally: outcomes and tallies (int64 [MATCH_TALLIES]) of the games that ended this turn; freezes the
+    truncated ones."""
+    import torch
+
+    dev, n = _device(), hi.shape[0]
+    rc = load().narde_match_tally(
+        _ptr(hi, torch.uint8, "hi", dev, (n, 16)), _ptr(done, torch.uint8, "done", dev, (n,)),
+        _ptr(truncated, torch.uint8, "truncated", dev, (n,)), n, env_base, _ptr(outcome, torch.uint8, "outcome", dev, (n,)),
+        _ptr(tallies, torch.int64, "tallies", dev, (MATCH_TALLIES,)), _stream())
+    _check(rc, "narde_match_tally")
 
 
 def step_chosen(lo, hi, env_base, seed, step, dice, choice, actions, counts, act_override=None, chosen=None, obs198=None,

@@ -18,6 +18,7 @@ namespace narde { __device__ int g_dbg_flags = 0; }
 #include "narde_deferred.cuh"
 #include "narde_env.cuh"
 #include "narde_lookahead.cuh"
+#include "narde_match.cuh"
 
 using namespace narde;
 
@@ -867,7 +868,7 @@ __device__ __forceinline__ int sample_prologue(const SampleArgs& S, int64_t i, i
   if (c == 0) return -1;
   const uint32_t below = (uint32_t)(S.params[0] * 16777216.0f);  // floor(eps * 2^24), exact for eps in [0, 1]
   if ((stream_random(S.seed, *env, *step, 2u).x >> 8) >= below) return -1;
-  return (int)mulhi32(turn_random(S.seed, *env, *step).z, (uint32_t)c);
+  return uniform_pick(S.seed, *env, *step, c);
 }
 // One env's segment as both segment kernels begin it: the count (clamped to cap), the first row, the sign (mode 1: BLACK
 // minimises) and, when sampling, the env's global id, the turn number and 1 / temperature.
@@ -888,11 +889,7 @@ __device__ __forceinline__ bool segment_begin(Segment& g, const float* score, co
   const int c = counts[i];
   g.c = c < cap ? c : cap;
   g.base = offsets[i];
-  g.sign = 1.0f;
-  if (mode == 1) {
-    const uint32_t meta = hi[i].z;
-    if ((int)(int8_t)((meta >> 16) & 0xFF) != 1) g.sign = -1.0f;
-  }
+  g.sign = mode == 1 ? rule_sign(mode, hi[i].z) : 1.0f;
   g.env = 0;
   g.step = 0;
   g.inv_tau = 0.0f;
@@ -909,14 +906,7 @@ __device__ __forceinline__ bool segment_begin(Segment& g, const float* score, co
   }
   return true;
 }
-// The order of the choice rule (include/narde_b200.h, narde_segment_argmax), shared by both segment kernels, their
-// shuffle reduction and the Gumbel path: (v, k) beats the current (best, best_k) when there is no current choice yet
-// (best_k == kNoChoice), or v is a number and best is NaN, or v > best, or v == best at a lower index.  A NaN never
-// beats a number, so one diverged afterstate does not decide the move, and an all-NaN segment keeps its first index.
-constexpr int kNoChoice = 0x7FFFFFFF;
-__device__ __forceinline__ bool beats(float v, int k, float best, int best_k) {
-  return best_k == kNoChoice || (!isnan(v) && (isnan(best) || v > best || (v == best && k < best_k)));
-}
+// (The order of the choice rule, beats(), is in narde_match.cuh: narde_match_choose uses it too.)
 
 // Gumbel noise of action k: u = ((w >> 9) + 1/2) / 2^23 lies strictly inside (0, 1) in float32, so G is finite
 __device__ __forceinline__ float gumbel(uint64_t seed, uint32_t env, uint64_t step, int k) {
@@ -1029,7 +1019,7 @@ __device__ __forceinline__ int64_t topk_begin(const TopkArgs& A, int64_t i, int*
   const int cnt = A.counts[i];
   *c = cnt < A.cap ? cnt : A.cap;
   *base = A.offsets[i];
-  *sign = (A.mode == 1 && (int)(int8_t)((A.hi[i].z >> 16) & 0xFF) != 1) ? -1.0f : 1.0f;
+  *sign = A.mode == 1 ? rule_sign(A.mode, A.hi[i].z) : 1.0f;
   return e;
 }
 __device__ __forceinline__ void topk_store(const TopkArgs& A, int64_t i, int64_t e, int64_t base, int j, int k) {
@@ -1165,6 +1155,156 @@ __global__ void __launch_bounds__(kThreads) k_lookahead_reduce(const uint4* hi, 
     if (act_override) act_override[i] = k >= cap ? cand_act[i * K + best] : 0ull;
   }
   if (any_unfit && uncovered) atomicAdd(uncovered, 1);
+}
+
+// ---- lock-step matches between two policies (narde_match.cuh; the rules: include/narde_b200.h) ----------------------
+// Per slot: its env (env_idx: a side batch's slot -> env, -1 = unused; NULL: slot i is env i) and its owner's count in
+// the owner's pool, 0 in the other and for a random owner.
+__global__ void __launch_bounds__(kThreads) k_match_split_counts(const uint4* hi, const int32_t* counts, int64_t n, int64_t env_base,
+                                                                const int32_t* env_idx, int kinds, int32_t* counts_a,
+                                                                int32_t* counts_b) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int64_t e = env_idx ? env_idx[i] : i;
+  int32_t ca = 0, cb = 0;
+  if (e >= 0) match_split((uint64_t)(env_base + e), hi[i].z, counts[i], kinds, &ca, &cb);
+  if (counts_a) counts_a[i] = ca;
+  if (counts_b) counts_b[i] = cb;
+}
+
+struct MatchArgs {
+  const uint4* hi;
+  const int32_t* counts;  // the legal counts (a random owner's list)
+  int64_t n;
+  int cap;
+  int64_t env_base;
+  const int32_t* env_idx;
+  uint64_t seed, step;
+  const uint64_t* step_dev;
+  int kinds;                     // bit p: seat p is a net
+  int mode[2];
+  const float* score[2];         // per seat: its pool's scores, each env's segment at offsets[e], counts_eff[e] long
+  const int64_t* offsets[2];
+  const int32_t* counts_eff[2];
+  int32_t* choice;
+  float* value;
+  int32_t* eff;
+};
+// The slot's env, owner and segment; returns false for an unused slot.  A random owner is settled here: k = (z * c) >> 32
+// over c = min(count, cap) (the `writer` thread stores it), and *net is false.
+__device__ __forceinline__ bool match_begin(const MatchArgs& A, int64_t i, bool writer, bool* net, int* c, int64_t* base,
+                                            float* sign, const float** score, int* p) {
+  const int64_t e = A.env_idx ? A.env_idx[i] : i;
+  if (e < 0) return false;
+  const uint64_t g = (uint64_t)(A.env_base + e);
+  const uint32_t meta = A.hi[i].z;
+  *p = match_owner(g, meta);
+  *net = (A.kinds >> *p) & 1;
+  if (!*net) {
+    const int cnt = A.counts[i];
+    const int cc = cnt < A.cap ? cnt : A.cap;
+    if (writer) {
+      const uint64_t step = A.step_dev ? *A.step_dev : A.step;
+      A.choice[i] = cc > 0 ? uniform_pick(A.seed, (uint32_t)g, step, cc) : 0;
+      A.value[i] = 0.0f;
+      if (A.eff) A.eff[i] = cc;
+    }
+    return true;
+  }
+  const int ce = A.counts_eff[*p][i];
+  *c = ce < A.cap ? ce : A.cap;
+  *base = A.offsets[*p][i];
+  *sign = rule_sign(A.mode[*p], meta);
+  *score = A.score[*p];
+  return true;
+}
+__device__ __forceinline__ void match_store(const MatchArgs& A, int64_t i, int c, const float* score, int64_t base, int best_k) {
+  A.choice[i] = c ? best_k : 0;
+  A.value[i] = c ? score[base + best_k] : 0.0f;
+  if (A.eff) A.eff[i] = c;
+}
+
+// A thread per env (cap <= 128): the owner's rule over the owner's segment.
+__global__ void __launch_bounds__(kThreads) k_match_choose(MatchArgs A) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= A.n) return;
+  bool net;
+  int c = 0, p = 0;
+  int64_t base = 0;
+  float sign = 1.0f;
+  const float* score = nullptr;
+  if (!match_begin(A, i, true, &net, &c, &base, &sign, &score, &p) || !net) return;
+  int best_k = kNoChoice;
+  float best = 0.0f;
+  for (int k = 0; k < c; k++) {
+    const float v = sign * score[base + k];
+    if (beats(v, k, best, best_k)) {
+      best = v;
+      best_k = k;
+    }
+  }
+  match_store(A, i, c, score, base, best_k);
+}
+
+// A warp per env (long lists: the side batch), lanes striding over the segment, as k_segment_argmax_warp.
+__global__ void __launch_bounds__(kThreads) k_match_choose_warp(MatchArgs A) {
+  const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (i >= A.n) return;  // (whole warps leave together)
+  bool net;
+  int c = 0, p = 0;
+  int64_t base = 0;
+  float sign = 1.0f;
+  const float* score = nullptr;
+  if (!match_begin(A, i, lane == 0, &net, &c, &base, &sign, &score, &p) || !net) return;
+  float best = 0.0f;
+  int best_k = kNoChoice;
+  for (int k = lane; k < c; k += 32) {
+    const float v = sign * score[base + k];
+    if (beats(v, k, best, best_k)) {
+      best = v;
+      best_k = k;
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_down_sync(0xFFFFFFFFu, best, o);
+    const int ok = __shfl_down_sync(0xFFFFFFFFu, best_k, o);
+    if (ok != kNoChoice && beats(ov, ok, best, best_k)) {
+      best = ov;
+      best_k = ok;
+    }
+  }
+  if (lane == 0) match_store(A, i, c, score, base, best_k);
+}
+
+// After narde_step_chosen: a running game (outcome 0) that terminated or was truncated this turn gets its outcome and is
+// added to the tallies (a warp-level reduction, one atomic per warp and non-zero slot); a truncated game is frozen
+// (FLAG_DONE), so that later turns leave it as it is.
+__global__ void __launch_bounds__(kThreads) k_match_tally(uint4* hi, const uint8_t* done, const uint8_t* truncated, int64_t n,
+                                                         int64_t env_base, uint8_t* outcome, int64_t* tallies) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int v[kMatchTallies] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  if (i < n && outcome[i] == MO_RUNNING && (done[i] || truncated[i])) {
+    const uint64_t g = (uint64_t)(env_base + i);
+    uint4 h = hi[i];
+    const int code = match_outcome(g, h.z, done[i] != 0, truncated[i] != 0);
+    outcome[i] = (uint8_t)code;
+    match_tally_add(g, code, (int)(h.w & 0xFFFF), v);
+    if (!done[i]) {
+      h.z |= FLAG_DONE << 24;
+      hi[i] = h;
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+    for (int k = 0; k < kMatchTallies; k++) v[k] += __shfl_xor_sync(0xFFFFFFFFu, v[k], o);
+  if ((threadIdx.x & 31) == 0) {
+#pragma unroll
+    for (int k = 0; k < kMatchTallies; k++)
+      if (v[k]) atomicAdd(reinterpret_cast<unsigned long long*>(tallies + k), (unsigned long long)v[k]);
+  }
 }
 
 // Trainer-compatible action codes (train_deepq_pytorch.py:432-437,495-507,752-761): for every stored legal
@@ -1592,6 +1732,42 @@ int narde_lookahead_reduce(const void* hi, const int32_t* cand_idx, const float*
   k_lookahead_reduce<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>(
       (const uint4*)hi, cand_idx, cand_score, (const uint4*)cand_hi, cand_act, cand_count, n, k, cap, reply_value, reply_count,
       reply_eff, choice, value, act_override, cand_value, uncovered);
+  return launch_status();
+}
+
+int narde_match_split_counts(const void* hi, const int32_t* counts, int64_t n, int64_t env_base, const int32_t* env_idx,
+                             int32_t kinds, int32_t* counts_a, int32_t* counts_b, void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || kinds < 0 || kinds > 3 || !hi || !counts || !aligned16(hi)) return -1;
+  if (((kinds & 1) && !counts_a) || ((kinds & 2) && !counts_b)) return -1;
+  k_match_split_counts<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>((const uint4*)hi, counts, n, env_base, env_idx, kinds,
+                                                                           counts_a, counts_b);
+  return launch_status();
+}
+
+int narde_match_choose(const void* hi, const int32_t* counts, int64_t n, int32_t cap, int64_t env_base, const int32_t* env_idx,
+                       uint64_t seed, uint64_t step, const uint64_t* step_dev, int32_t kinds, int32_t mode_a, int32_t mode_b,
+                       const float* score_a, const int64_t* offsets_a, const int32_t* counts_eff_a, const float* score_b,
+                       const int64_t* offsets_b, const int32_t* counts_eff_b, int32_t* choice, float* value, int32_t* eff,
+                       void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || cap <= 0 || kinds < 0 || kinds > 3 || !hi || !counts || !choice || !value || !aligned16(hi)) return -1;
+  if ((kinds & 1) && (!score_a || !offsets_a || !counts_eff_a || (mode_a != 0 && mode_a != 1))) return -1;
+  if ((kinds & 2) && (!score_b || !offsets_b || !counts_eff_b || (mode_b != 0 && mode_b != 1))) return -1;
+  const MatchArgs A = {(const uint4*)hi, counts, n, cap, env_base, env_idx, seed, step, step_dev, kinds, {mode_a, mode_b},
+                       {score_a, score_b}, {offsets_a, offsets_b}, {counts_eff_a, counts_eff_b}, choice, value, eff};
+  if (cap > 128)  // long segments: a warp per env, as launch_segment
+    k_match_choose_warp<<<grid_for(n * 32), kThreads, 0, (cudaStream_t)stream>>>(A);
+  else
+    k_match_choose<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>(A);
+  return launch_status();
+}
+
+int narde_match_tally(void* hi, const uint8_t* done, const uint8_t* truncated, int64_t n, int64_t env_base, uint8_t* outcome,
+                      int64_t* tallies, void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || !hi || !done || !truncated || !outcome || !tallies || !aligned16(hi) || (((uintptr_t)tallies) & 7u) != 0) return -1;
+  k_match_tally<<<grid_for(n), kThreads, 0, (cudaStream_t)stream>>>((uint4*)hi, done, truncated, n, env_base, outcome, tallies);
   return launch_status();
 }
 

@@ -357,6 +357,47 @@ int narde_lookahead_reduce(const void *hi, const int32_t *cand_idx, const float 
                            int32_t *choice, float *value, uint64_t *act_override, float *cand_value,
                            int32_t *uncovered, void *stream);
 
+/* Lock-step matches between two policies A and B (gym_narde_b200.AfterstateMatch), each an afterstate net or the random
+ * agent.  Seats: in game g (the global env id env_base + i) A plays WHITE when g is even and BLACK when g is odd; the seat
+ * whose colour is to move owns the env's turn.  kinds: bit 0 set = A is a net, bit 1 = B is a net.
+ * A net owner plays narde_segment_argmax's choice in its mode (0 or 1) over its own scores; a random owner plays
+ * k = (z * c) >> 32 over c = min(count, cap), z = word z of Philox stream 0 (see narde_segment_sample): over the whole list
+ * exactly the uniform action of narde_step_full.  Every afterstate row is scored once, by the owner's net.
+ *
+ * narde_match_split_counts: counts_a[i] = counts[i] when A is a net and owns env i's turn, else 0; counts_b likewise (a
+ * count array of a random seat may be NULL).  env_idx (may be NULL): [n] i32, slot i holds env env_idx[i] (g = env_base +
+ * env_idx[i]; a side batch of narde_gather_overflow), -1 = unused slot (both counts 0).  hi: the slots' states. */
+int narde_match_split_counts(const void *hi, const int32_t *counts, int64_t n, int64_t env_base, const int32_t *env_idx,
+                             int32_t kinds, int32_t *counts_a, int32_t *counts_b, void *stream);
+/* narde_match_choose: for slot i (env_idx as above; unused slots are not written), owner p:
+ *   - p random: choice[i] = (z * c) >> 32 with c = min(counts[i], cap) (0 when c == 0), value[i] = 0, eff[i] = c;
+ *   - p a net: narde_segment_argmax's rule in mode_p over score_p[offsets_p[i] + k], k < c = min(counts_eff_p[i], cap):
+ *     choice[i] = its index, value[i] = its score (0, 0 when c == 0), eff[i] = c -- the length of the prefix the choice was
+ *     made from, 0 when the owner's rows did not fit its pool: the sub_counts_eff narde_scatter_choice takes.
+ * A net seat's score / offsets / counts_eff must be given, a random seat's may be NULL; eff may be NULL.  step_dev (may be
+ * NULL) overrides `step` with the device-resident turn number.  A thread per env for cap <= 128, a warp per env above. */
+int narde_match_choose(const void *hi, const int32_t *counts, int64_t n, int32_t cap, int64_t env_base, const int32_t *env_idx,
+                       uint64_t seed, uint64_t step, const uint64_t *step_dev, int32_t kinds, int32_t mode_a, int32_t mode_b,
+                       const float *score_a, const int64_t *offsets_a, const int32_t *counts_eff_a, const float *score_b,
+                       const int64_t *offsets_b, const int32_t *counts_eff_b, int32_t *choice, float *value, int32_t *eff,
+                       void *stream);
+/* narde_match_tally, after narde_step_chosen (done / truncated: its outputs): env i with outcome[i] == 0 that terminated or
+ * was truncated this turn gets outcome[i] = 1 (A won), 2 (B won) or 3 (truncated), + 4 for a mars: the winner is the side
+ * with 15 checkers off, a mars is the loser having none off.  A truncated game is frozen (FLAG_DONE set in its state) so
+ * that later turns leave it as it is.  Each new outcome adds to tallies[NARDE_MATCH_TALLIES] (int64, caller zeroes): */
+#define NARDE_MATCH_GAMES 0
+#define NARDE_MATCH_A_WINS 1
+#define NARDE_MATCH_B_WINS 2
+#define NARDE_MATCH_A_MARS 3       /* A's wins by mars */
+#define NARDE_MATCH_B_MARS 4
+#define NARDE_MATCH_TRUNCATED 5
+#define NARDE_MATCH_A_WHITE_WINS 6 /* A's wins as WHITE (even g) */
+#define NARDE_MATCH_B_WHITE_WINS 7 /* B's wins as WHITE (odd g) */
+#define NARDE_MATCH_PLIES 8        /* the summed episode steps of the games, truncated ones included */
+#define NARDE_MATCH_TALLIES 9
+int narde_match_tally(void *hi, const uint8_t *done, const uint8_t *truncated, int64_t n, int64_t env_base, uint8_t *outcome,
+                      int64_t *tallies, void *stream);
+
 /* Trainer-compatible action codes for every stored legal turn action: the reference's (move1_code,
  * move2_code) pairs (train_deepq_pytorch.py:432-437,495-507; action_to_idx :752-761): code = from*24 + to,
  * to = 0 for a bear-off, move2_code = 0 when the turn has a single half-move.  codes: [n,cap,3] i32 =
